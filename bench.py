@@ -2,13 +2,17 @@
 """Benchmark of the bridge hot path (BASELINE.json metric: bridge fwd+bwd samples/s; caption decode
 tokens/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 One "step" = one forward + backward of the bridge over one synthetic batch of config C2
 (B=8 per GPU, L=128 text tokens, Nv=257 vision tokens, vision 1024 -> language 2304, 2 blocks,
 heads 8/18, train mode with dropout 0.1 as `FullModel` builds it, full_model.py:38,72), upstream
 gradient of loss = mean(y^2) (SURVEY.md 8d), bf16 weight copies refreshed every step as after an
 optimizer update. Prints ONE JSON line (rank 0). See DESIGN.md "Measurement" for every field.
+
+--dump-outputs DIR writes what the last timed step of the CUDA-graph replay (of the eager launches under
+--no-graph) handed its caller, the loss and every parameter's gradient, as DIR/<name>.npy. Inputs, weights
+and dropout seeds are fixed, so two builds run with the same arguments can be compared array for array.
 """
 from __future__ import annotations
 
@@ -21,6 +25,7 @@ import sys
 import tempfile
 import threading
 import time
+import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
@@ -55,6 +60,27 @@ def decode_bytes_per_step(B: int, s: int, Nv: int, position_rows: bool = False) 
     D = D_LANG
     lens = [1 if (position_rows and i == 0) else s for i in range(N_BLOCKS)]
     return sum(B * 2.0 * Nv * D * 2 + 2.0 * B * lq * D * 2 for lq in lens)
+
+
+DUMP_ELEMS = 1 << 18   # per array: at most 52 x 1 MB of float32 in all
+
+
+def step_outputs(loss, named_params) -> dict:
+    """What one bridge step hands its caller, as float32 host arrays for --dump-outputs: the loss and the
+    gradient of every parameter. A gradient of more than DUMP_ELEMS elements is sampled at DUMP_ELEMS flat
+    positions drawn from a seed derived from the parameter's name, so every run samples the same positions."""
+    import numpy as np
+    import torch
+
+    out = {"loss": loss.detach().float().reshape(1).cpu().numpy()}
+    for name, p in named_params:
+        g = p.grad.detach().reshape(-1)
+        if g.numel() > DUMP_ELEMS:
+            rng = np.random.default_rng(zlib.crc32(name.encode()))
+            idx = np.sort(rng.choice(g.numel(), DUMP_ELEMS, replace=False))
+            g = g[torch.from_numpy(idx).to(g.device)]
+        out["grad." + name] = g.float().cpu().numpy()
+    return out
 
 
 def load_peaks() -> dict:
@@ -354,7 +380,13 @@ def run_b200_arm(args) -> int:
     if rank == 0:
         sampler.start()
 
-    def timed_loop(fn):
+    # --dump-outputs takes the last timed step of the launch mode the arguments fix: the graph replay, or the eager
+    # launches under --no-graph (or when capture failed). Not the faster mode of the run: the two modes draw different
+    # dropout seeds, and which one is faster can change from build to build.
+    dump_mode = "eager launches" if graphed is None else "cuda graph replay (GraphedBridgeStep)"
+    outputs = {}
+
+    def timed_loop(fn, mode):
         for _ in range(max(3, args.warmup)):
             fn()
         sync_all()
@@ -363,10 +395,13 @@ def run_b200_arm(args) -> int:
         a.record()
         t0 = time.perf_counter()
         for _ in range(args.steps):
-            fn()
+            loss = fn()
         host_ms = (time.perf_counter() - t0) * 1e3 / args.steps   # time to ENQUEUE a step (no sync inside)
         b.record()
         sync_all()
+        if args.dump_outputs and mode == dump_mode:   # before the next loop overwrites them
+            model.materialize_grads()      # N > 1: the averaged weight gradients out of the bf16 arena
+            outputs[mode] = step_outputs(loss, model.named_parameters())
         ms = a.elapsed_time(b)
         if world > 1:                                              # a mode is as fast as its slowest rank
             tt_ = torch.tensor([ms], device=dev, dtype=torch.float64)
@@ -380,13 +415,20 @@ def run_b200_arm(args) -> int:
     sampler.mark(True)
     modes = {}
     if graphed is not None:
-        ms_g, host_g, _ = timed_loop(lambda: graphed.replay())
-        modes["cuda graph replay (GraphedBridgeStep)"] = (ms_g, host_g, graphed.kernels_per_replay * args.steps)
+        mode = "cuda graph replay (GraphedBridgeStep)"
+        ms_g, host_g, _ = timed_loop(lambda: graphed.replay(), mode)
+        modes[mode] = (ms_g, host_g, graphed.kernels_per_replay * args.steps)
     if graphed is None or not args.graph_only:
-        modes["eager launches"] = timed_loop(lambda: step(vision_d, text_d))
+        modes["eager launches"] = timed_loop(lambda: step(vision_d, text_d), "eager launches")
     sampler.mark(False)
     best_mode = min(modes, key=lambda k: modes[k][0])
     ms_total, host_ms_step, launches = modes[best_mode]
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in outputs[dump_mode].items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     if best_mode == "eager launches":
         graphed_for_e2e, graphed = graphed, None                 # e2e and the dp leg follow the headline mode
     # ---- end-to-end: host buffers in, loss out, through the public nn.Module API ---------------
@@ -1199,7 +1241,15 @@ def main() -> int:
     ap.add_argument("--workload", default="c2", choices=["c2", "c5"],
                     help="c2 = BASELINE.json configs[1] (the headline, default); c5 = the 518 px stress config "
                          "(batch 16, 1370 vision tokens), bridge fwd+bwd only")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and the parameter gradients of the last timed graph replay (eager step under "
+                         "--no-graph) as DIR/<name>.npy (float32; "
+                         f"gradients of more than {DUMP_ELEMS} elements sampled at fixed seeded positions)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     if args.workload == "c5":
         global B_PER_GPU, N_VIS, WORKLOAD
         B_PER_GPU, N_VIS, WORKLOAD = 16, 1370, "C5"

@@ -1,9 +1,11 @@
 """bench.py prints ONE JSON line on stdout whatever libraries write to fd 1 (NCCL prints its version
-banner there on some boxes); host-side helpers of the bench (no GPU needed)."""
+banner there on some boxes); host-side helpers of the bench (no GPU needed); --dump-outputs end to end (GPU)."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -56,6 +58,54 @@ def test_decode_gemm_flops_and_workload_config():
     assert "gradients" not in c1 and c1["parallelism"] == "single" and c1["global_batch"] == 8
     assert "bf16 arena" in c8["gradients"] and c8["parallelism"] == "dp8" and c8["global_batch"] == 64
     assert "model" not in c1 and c1["workload"].startswith("C2")
+
+
+def test_dumped_outputs_are_float32_bounded_and_sampled_at_fixed_positions():
+    """--dump-outputs: the loss and every gradient as float32; a large gradient is sampled at the same positions in
+    every run, and the bridge's 52 gradients stay under 64 MB in all."""
+    import numpy as np
+    import torch
+
+    sys.path.insert(0, ROOT)
+    import bench
+
+    assert 52 * bench.DUMP_ELEMS * 4 <= 64 << 20
+    m = torch.nn.Linear(bench.DUMP_ELEMS // 256 + 1, 512)
+    m(torch.randn(3, m.in_features)).square().mean().backward()
+    loss = torch.tensor(1.25)
+    a = bench.step_outputs(loss, m.named_parameters())
+    b = bench.step_outputs(loss, m.named_parameters())
+    assert sorted(a) == ["grad.bias", "grad.weight", "loss"]
+    assert all(v.dtype == np.float32 for v in a.values()) and a["loss"].tolist() == [1.25]
+    assert np.array_equal(a["grad.bias"], m.bias.grad.numpy())
+    w = m.weight.grad.reshape(-1).numpy()
+    assert a["grad.weight"].shape == (bench.DUMP_ELEMS,) and np.array_equal(a["grad.weight"], b["grad.weight"])
+    assert np.isin(a["grad.weight"], w).all()
+
+
+@pytest.mark.gpu
+@pytest.mark.timeout(900)
+def test_dump_outputs_are_identical_from_run_to_run(tmp_path):
+    """bench.py --dump-outputs run twice with the same arguments writes the same arrays, in the default launch mode
+    (graph replay) and under --no-graph (eager launches, which draw their dropout seeds differently)."""
+    import numpy as np
+
+    legs = ["--no-cpu-baseline", "--no-decode", "--no-train-step", "--no-inloop"]
+
+    def run(name, *extra):
+        out = tmp_path / name
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", "3", "--warmup", "1",
+                            *legs, *extra, "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-3000:]
+        assert json.loads(r.stdout)["steps"] == 3
+        return {f: np.load(out / f) for f in sorted(os.listdir(out))}
+
+    for extra in ((), ("--no-graph",)):
+        a, b = run("a" + "".join(extra), *extra), run("b" + "".join(extra), *extra)
+        assert len(a) == 53 and "loss.npy" in a and list(a) == list(b)
+        assert all(v.dtype == np.float32 and np.isfinite(v).all() for v in a.values())
+        assert sum(v.nbytes for v in a.values()) <= 64 << 20
+        assert [f for f in a if not np.array_equal(a[f], b[f])] == [], extra
 
 
 def test_torch_library_arm_is_the_same_arithmetic():

@@ -2,18 +2,18 @@
 round-trip, files are exchangeable with the reference module in both directions, only rank 0 writes
 under data parallelism. Host-side logic: runs without a GPU (the flat-arena snapshot path is covered by
 the `gpu` test at the bottom)."""
-import importlib.util
 import os
 import pathlib
 import sys
 
+import numpy as np
 import pytest
 import torch
 
 from oracle import bridge_oracle as O
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/src/vlm_bridge/model_architecture/bridge_module.py"
+GOLDEN = os.path.join(ROOT, "tests", "golden", "tiny_bridge.npz")
 TINY = dict(vision_dim=32, language_dim=64, num_blocks=2, num_heads_cross=2, num_heads_self=1)
 
 
@@ -102,22 +102,35 @@ def test_untrusted_pickles_are_refused_unless_asked(tmp_path):
     assert not [f for f in os.listdir(tmp_path) if ".tmp." in f]               # atomic rename, nothing left behind
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference tree only exists in the build container")
+def _reference_bridge():
+    """The reference `BridgeLite` at the TINY widths as its checkpoint files see it: the reference module's own
+    state_dict, stored in tests/golden/tiny_bridge.npz by make_golden.py, as parameters under the same names, in
+    the same registration order and with the same shapes."""
+    z = np.load(GOLDEN)
+    bridge = torch.nn.Module()
+    for key in z.files:
+        if not key.startswith("param/"):
+            continue
+        *path, leaf = key[len("param/"):].split(".")
+        mod = bridge
+        for part in path:
+            if part not in mod._modules:
+                mod.add_module(part, torch.nn.Module())
+            mod = mod._modules[part]
+        mod.register_parameter(leaf, torch.nn.Parameter(torch.from_numpy(z[key])))
+    assert list(bridge.state_dict()) == O.param_names(2)
+    return bridge
+
+
 def test_files_are_exchangeable_with_the_reference_module(tmp_path):
     from vlm_bridge_b200 import checkpoint as ck
-
-    spec = importlib.util.spec_from_file_location("ref_bridge_module", REF)
-    ref_mod = importlib.util.module_from_spec(spec)
-    sys.dont_write_bytecode = True
-    spec.loader.exec_module(ref_mod)
 
     class FullModelLike(torch.nn.Module):                                      # the prefix FullModel gives (full_model.py:68)
         def __init__(self, bridge):
             super().__init__()
             self.bridge_module = bridge
 
-    torch.manual_seed(7)
-    ref = ref_mod.BridgeLite(dropout=0.1, **TINY)
+    ref = _reference_bridge()
     # reference -> here, Format A (FullModel.save_model) and Format B (save_checkpoint)
     torch.save({"bridge_module_state_dict": ref.state_dict(), "model_config": {}}, tmp_path / "ref_a.pth")
     ref_opt = torch.optim.AdamW(ref.parameters(), lr=1e-5, weight_decay=0.01)
@@ -137,7 +150,7 @@ def test_files_are_exchangeable_with_the_reference_module(tmp_path):
     opt.step()
     ck.save_checkpoint(str(tmp_path), mine, opt, epoch=5, is_best=True, asynchronous=False)
     ckpt = torch.load(tmp_path / "latest_checkpoint.pth")
-    ref2 = FullModelLike(ref_mod.BridgeLite(dropout=0.1, **TINY))
+    ref2 = FullModelLike(_reference_bridge())
     msd = ref2.state_dict()
     for k, v in ckpt["model_state_dict"].items():
         assert k in msd

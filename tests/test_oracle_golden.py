@@ -1,19 +1,17 @@
 """The oracle is only as good as its pin: check it against fixtures generated from the unmodified
-reference module (tests/golden/make_golden.py), and against the reference itself when it is
-present (build container only)."""
-import importlib.util
+reference module (tests/golden/make_golden.py), and against the reference itself where a copy of it
+sits in oracle/_ref (oracle/make_ref.py)."""
 import json
 import os
-import sys
 
 import numpy as np
 import pytest
 import torch
 
 from oracle import bridge_oracle as O
+from oracle import make_ref
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = "/root/reference/src/vlm_bridge/model_architecture/bridge_module.py"
 
 
 def _rel(a, b, floor=1e-2):
@@ -108,12 +106,9 @@ def test_full_backward_fingerprint(full_fp, full_run):
         assert abs(float(grads[k].norm()) - v) <= 2e-4 * v + 1e-9, k
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference tree only exists in the build container")
+@pytest.mark.skipif(make_ref.bridge_module_path() is None, reason="no copy of the reference module in oracle/_ref")
 def test_against_live_reference_module():
-    sys.dont_write_bytecode = True
-    spec = importlib.util.spec_from_file_location("ref_bridge_module", REF)
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
+    ref = make_ref.load_reference_bridge_module()
     cfg = dict(vision_dim=48, language_dim=96, num_blocks=3, num_heads_cross=2, num_heads_self=3)
     torch.manual_seed(5)
     m = ref.BridgeLite(dropout=0.0, **cfg).eval()
