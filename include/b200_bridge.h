@@ -56,6 +56,14 @@ const char* b200b_profile_entry(int index, float* ms);
 /* ------------------------------------------------------------------------------------------- *
  * Dropout: Philox4x32-10 keyed by `seed`; each fused op below names the `stream` id it uses so
  * forward and backward regenerate identical masks. p == 0 disables.
+ * GEMM epilogues and casts: element i (row-major position row * n + col of the logical [m, n] result,
+ * independent of the row pitch and the tile configuration) is kept iff the 16-bit lane i % 8 of
+ * Philox4x32-10(counter = (i / 8 low, i / 8 high, stream, 0x0b200b00), key = (seed low, seed high))
+ * is >= round(p * 65536); kept values are scaled by 1 / (1 - p) after their bf16 rounding.
+ * Non-finite values: a kept inf / NaN propagates; a dropped position is an exact 0 (the residual
+ * epilogue adds nothing), whatever its value -- unlike torch's x * mask, which turns a dropped inf
+ * into NaN. The dGELU epilogue still multiplies the dropped 0 by gelu'(aux), so a non-finite aux
+ * gives NaN there, as in torch.
  * Replaces nn.Dropout / SDPA dropout_p (bridge_module.py:137,235,294,296).
  * ------------------------------------------------------------------------------------------- */
 
@@ -500,7 +508,9 @@ int b200b_allreduce_nvls(const b200b_nvls_comm* comm, int dtype, int64_t byte_of
 /* Number of SMs the persistent compute kernels of this library (the tcgen05 GEMMs) may occupy on the
  * calling thread's current device: min(limit, SMs of the device); 0 or negative removes the limit.
  * The data-parallel path lowers it by the SMs it reserves for the gradient exchange, so that the
- * statically scheduled GEMM CTAs never share (or wait for) an SM with an exchange CTA. Process-wide. */
+ * statically scheduled GEMM CTAs never share (or wait for) an SM with an exchange CTA. Process-wide.
+ * A CTA pair (cta_group 2) needs two SMs: under a limit of 1 the GEMMs run single-CTA tiles, and
+ * b200b_gemm_dual runs its two launches. Results do not depend on the limit. */
 void b200b_set_sm_limit(int sms);
 int b200b_get_sm_limit(void);
 

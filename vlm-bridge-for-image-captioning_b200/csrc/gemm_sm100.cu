@@ -925,7 +925,7 @@ TileChoice choose_tile(int m, int n, int num_sms) {
   // CTA pairs beat single CTAs on every bridge shape measured (profiles/r01_gemm_tile_sweep.jsonl);
   // the width is chosen by counting waves of pair tiles over the num_sms/2 pairs. 128-wide tiles
   // sustain ~88% of the 256-wide main-loop rate.
-  const long long units = num_sms / 2;
+  const long long units = num_sms >= 2 ? num_sms / 2 : 1;
   double best = 1e300;
   TileChoice out{2, 256};
   const int widths[2] = {256, 128};
@@ -1001,6 +1001,9 @@ extern "C" int b200b_gemm(const b200b_gemm_args* a, void* stream_) {
     set_last_error("gemm: block_n must be 0, 128 or 256 and cta_group 0, 1 or 2");
     return B200B_ERR_ARG;
   }
+  // A CTA pair occupies two SMs. Under an SM limit of 1 the tiles run on single CTAs instead: the
+  // per-element k order is the same, so the result is too.
+  if (num_sms < 2) cta_group = 1;
   const bool pair = cta_group == 2;
   // rows of the B tile one CTA stages: the whole tile, or half of it in a CTA pair
   const int b_rows = pair ? block_n / 2 : block_n;
@@ -1098,9 +1101,9 @@ extern "C" int b200b_gemm_dual(const b200b_gemm_args* dgrad, const b200b_gemm_ar
   if (rc != B200B_OK) return rc;
   // The grouped kernel covers exactly the pair it was written for: dgrad form (A K-major, B MN-major, bf16 out, no
   // bias) + wgrad form (A and B MN-major, fp32 or bf16 out, no bias, beta = 0), both on 256 x 128 pair tiles, no
-  // dropout. Anything else runs as the two launches it stands for.
+  // dropout, at least one CTA pair under the SM limit. Anything else runs as the two launches it stands for.
   const bool eligible =
-      b200b_gemm_set_dual(-1) != 0 && dgrad->a_major == 0 && dgrad->b_major == 1 && dgrad->epilogue == B200B_EPI_BF16_BIAS &&
+      b200b_gemm_set_dual(-1) != 0 && num_sms >= 2 && dgrad->a_major == 0 && dgrad->b_major == 1 && dgrad->epilogue == B200B_EPI_BF16_BIAS &&
       dgrad->bias == nullptr && wgrad->a_major == 1 && wgrad->b_major == 1 &&
       (wgrad->epilogue == B200B_EPI_F32 || wgrad->epilogue == B200B_EPI_BF16_BIAS) && wgrad->bias == nullptr &&
       wgrad->beta == 0.f && dgrad->dropout_p == 0.f && wgrad->dropout_p == 0.f && dgrad->block_n == 0 && wgrad->block_n == 0 &&
