@@ -450,6 +450,36 @@ int b200b_cross_entropy_bwd(const void* logits, int dtype, int64_t ld, const int
                             const float* out2, const float* grad_loss, void* dlogits, int64_t ldd,
                             void* stream);
 
+/* ------------------------------------------------------------------------------------------- *
+ * Temperature / top-p sampling, one token per row (csrc/sampling.cu). Replaces the sampling branch of a
+ * decode step of FullModel.generate_caption(do_sample=True) (full_model.py:264-350: NaN / Inf guards,
+ * logits / temperature, top-p filter, multinomial).
+ *
+ * logits [rows, vocab], row pitch ld >= vocab elements (nothing beyond vocab is read), dtype 0 = f32,
+ * 1 = bf16; arithmetic is fp32. For row b at decode step t:
+ *  1. guards (as the greedy decode): a row containing a NaN becomes all zeros; otherwise a row containing
+ *     +-Inf is clamped to [-100, 100];
+ *  2. z_i = x_i / temperature (fp32 division), temperature finite and > 0;
+ *  3. token i is kept iff the softmax(z) mass of the tokens with STRICTLY larger z is < top_p, top_p in
+ *     (0, 1]: the sort-and-cumsum nucleus rule, except that tokens tied at the threshold are kept together;
+ *     the maximum is always kept and top_p = 1 keeps every token;
+ *  4. ids_out[b * ids_stride] = argmax over kept i of z_i + g_i, g_i = -ln(-ln u_i) (Gumbel-max: an exact
+ *     draw from the renormalised nucleus), ties to the smallest index;
+ *  5. u_i = ((w >> 8) + 0.5) * 2^-24, w = 32-bit word i % 4 of Philox4x32-10(counter = (i / 4, b, t mod 2^32,
+ *     0x5a3b1e00), key = (seed low, seed high)); *seed is read from device memory when the kernel runs, so
+ *     a captured graph or a sync-free loop draws new values by changing it. The logs are accurate logf /
+ *     log1pf (u is carried exactly as u below 1/2 and as 1 - u above).
+ * The mass comparisons of 3 use exp(z - zmax) in 2^-40 fixed point (relative error of a mass below 2e-5).
+ * Limits: vocab <= 8 * (180224 / e) = 360448 (f32) / 720896 (bf16) tokens -- a row is split over a cluster
+ * of at most 8 CTAs holding 176 KiB of it each -- else B200B_ERR_SHAPE, as for rows < 1 or vocab < 1.
+ * B200B_ERR_ARG: a null pointer, dtype not 0 / 1, ld < vocab, temperature <= 0 or not finite, top_p
+ * outside (0, 1]. The cluster size is 1, 2, 4 or 8: the fewest CTAs the row fits, doubled while
+ * rows * CTAs is below the SM count and each CTA keeps >= 4096 tokens.
+ * ------------------------------------------------------------------------------------------- */
+int b200b_sample_tokens(const void* logits, int dtype, int64_t ld, int64_t rows, int64_t vocab, float temperature,
+                        float top_p, const unsigned long long* seed, int64_t step, int64_t* ids_out,
+                        int64_t ids_stride, void* stream);
+
 /* out f32 [n] = scale * in bf16 [n] (n % 8 == 0): turns an exchanged bf16 gradient bucket into
  * the fp32 .grad the optimizer reads. */
 int b200b_bf16_to_f32(const void* in_bf16, float* out, int64_t n, float scale, void* stream);

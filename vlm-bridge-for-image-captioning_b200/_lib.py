@@ -145,6 +145,9 @@ def _declare(lib) -> None:
     lib.b200b_cross_entropy_bwd.restype = C.c_int
     lib.b200b_cross_entropy_bwd.argtypes = ([C.c_void_p, C.c_int, C.c_int64, C.c_void_p] + [C.c_int64] * 4 +
                                             [C.c_void_p] * 4 + [C.c_int64, C.c_void_p])
+    lib.b200b_sample_tokens.restype = C.c_int
+    lib.b200b_sample_tokens.argtypes = [C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_int64, C.c_float, C.c_float,
+                                        C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]
     lib.b200b_gemm_dual.restype = C.c_int
     lib.b200b_gemm_dual.argtypes = [C.POINTER(GemmArgs), C.POINTER(GemmArgs), C.c_void_p]
     lib.b200b_gemm_set_dual.restype = C.c_int

@@ -1,11 +1,13 @@
-"""Batched greedy caption decode over a per-image cached vision K/V (SURVEY.md 8a row a12, 8f rank 2).
+"""Batched caption decode over a per-image cached vision K/V (SURVEY.md 8a row a12, 8f rank 2).
 
-Mirrors the greedy branch of `FullModel.generate_caption` (full_model.py:241-363, `do_sample=False`):
+Mirrors `FullModel.generate_caption` (full_model.py:241-363); the greedy branch (`do_sample=False`):
 start from BOS, every step embeds the whole prefix, runs the bridge over it (the bridge
 self-attention is non-causal, so earlier positions change when a token is appended and the prefix
 must be recomputed -- only the image's K/V are exactly cacheable), feeds the result to the language
 model, takes `argmax` of the last position's logits (NaN logits -> zeros, Inf logits -> clamped to
-+-100, as :270-283) and appends it.
++-100, as :270-283) and appends it. With `do_sample=True` the token is drawn instead (temperature, top-p
+nucleus, one fused kernel per step: `ops.sample_tokens`, csrc/sampling.cu), as the sampling branch
+(:264-350) does.
 
 The reference loop is batch-1 and synchronises with the host up to three times per step
 (`next_token.item()`, :317,355-366). Here B images decode together with no host synchronisation:
@@ -19,10 +21,12 @@ independent reference runs produce (generation is deterministic and rows never i
 """
 from __future__ import annotations
 
+import math
 from typing import Callable, Optional
 
 import torch
 
+from . import ops
 from .kv_cache import VisionKVCache
 
 __all__ = ["greedy_decode", "DecodeStepGraphs"]
@@ -81,7 +85,9 @@ def greedy_decode(bridge, vision_features: torch.Tensor, embed_fn: Callable[[tor
                   eos_token_id: Optional[int] = None, max_new_tokens: int = 50,
                   kv_cache: Optional[VisionKVCache] = None, use_cache: bool = True,
                   step_graphs: Optional[DecodeStepGraphs] = None, use_graphs: bool = False,
-                  cache_positions: bool = True, precision: str = "bf16", refill_cache: bool = False):
+                  cache_positions: bool = True, precision: str = "bf16", refill_cache: bool = False,
+                  do_sample: bool = False, temperature: float = 1.0, top_p: float = 1.0,
+                  generator: Optional[torch.Generator] = None):
     """Returns (ids [B, 1 + max_new_tokens] int64 incl. BOS, lengths [B] int64): row b's caption is
     ids[b, 1:lengths[b]] (EOS excluded); positions from lengths[b] on are what the lock-step loop kept
     generating and are to be ignored. `use_graphs` replays one captured CUDA graph of the bridge per
@@ -94,12 +100,35 @@ def greedy_decode(bridge, vision_features: torch.Tensor, embed_fn: Callable[[tor
     numerics (generate_caption runs without autocast, full_model.py:221-261), for which the token ids equal
     the fp32 reference's on every step; "bf16" is the tensor-core path (the reference's autocast numerics).
     `refill_cache=True` with a `kv_cache` from an earlier call recomputes that cache in place for
-    `vision_features` (same shape), so `step_graphs` captured over it are replayed for new images."""
+    `vision_features` (same shape), so `step_graphs` captured over it are replayed for new images.
+
+    `do_sample=True` draws each token instead of taking the argmax (generate_caption(do_sample=True)): per row,
+    the NaN / Inf guards above, z = logits / `temperature` (finite, > 0), the top-p nucleus (tokens whose
+    strictly-larger-z softmax mass is < `top_p`, top_p in (0, 1]; ties at the threshold are kept together), and
+    an exact draw from the renormalised nucleus (Gumbel-max over Philox4x32-10 of (seed, row, step); the rule is
+    stated in include/b200_bridge.h). One 64-bit seed per call is drawn on the device from `generator` (a CUDA
+    generator on the images' device; None = that device's default generator), so the loop never waits for the
+    host and the same generator state gives the same captions. The step graphs still capture only the bridge;
+    the sampler runs after each replay. Bad `temperature` / `top_p` values or a generator on another device
+    raise ValueError before any kernel runs."""
     was_training = bridge.training
     bridge.eval()
     try:
         B = vision_features.shape[0]
         dev = vision_features.device
+        if do_sample:
+            temperature, top_p = float(temperature), float(top_p)
+            if not (math.isfinite(temperature) and temperature > 0.0):
+                raise ValueError(f"temperature must be finite and > 0, got {temperature}")
+            if not (0.0 < top_p <= 1.0):
+                raise ValueError(f"top_p must be in (0, 1], got {top_p}")
+            if dev.type != "cuda":
+                raise ValueError("do_sample=True needs the images on a CUDA device")
+            gdev = None if generator is None else torch.device(generator.device)
+            if gdev is not None and gdev.type == "cuda" and gdev.index is None:
+                gdev = torch.device("cuda", torch.cuda.current_device())
+            if gdev is not None and gdev != dev:
+                raise ValueError(f"generator is on {generator.device}, the images on {dev}")
         if precision not in ("bf16", "fp32"):
             raise ValueError("precision must be 'bf16' or 'fp32'")
         if precision == "fp32" and not use_cache:
@@ -119,6 +148,8 @@ def greedy_decode(bridge, vision_features: torch.Tensor, embed_fn: Callable[[tor
             step_graphs = None
         ids = torch.empty((B, 1 + max_new_tokens), dtype=torch.long, device=dev)
         ids[:, 0] = bos_token_id
+        if do_sample:
+            seed = torch.empty(1, dtype=torch.int64, device=dev).random_(generator=generator)
         for step in range(max_new_tokens):
             prefix = ids[:, :step + 1]
             kpos = step if (cache_positions and use_cache) else None
@@ -130,6 +161,12 @@ def greedy_decode(bridge, vision_features: torch.Tensor, embed_fn: Callable[[tor
             logits = lm_fn(hidden)
             if logits.dim() == 3:
                 logits = logits[:, -1, :]
+            if do_sample:
+                if logits.dtype not in (torch.float32, torch.bfloat16) or logits.stride(-1) != 1:
+                    logits = logits.float().contiguous()
+                ops.sample_tokens(logits, temperature=temperature, top_p=top_p, seed=seed, step=step,
+                                  out=ids[:, step + 1])
+                continue
             logits = logits.float()
             # numerical guards of the reference, as tensor ops (no host sync)
             # (per row: the reference applies them to one caption at a time, full_model.py:270-283)

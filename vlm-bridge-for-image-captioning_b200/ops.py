@@ -279,6 +279,32 @@ def attention_decode_tc(q: torch.Tensor, kv_tc: torch.Tensor, *, block_index: in
     return out, lse
 
 
+def sample_tokens(logits: torch.Tensor, *, temperature: float, top_p: float, seed: torch.Tensor, step: int,
+                  out: torch.Tensor | None = None) -> torch.Tensor:
+    """One token per row of logits [rows, V] (fp32 or bf16, unit inner stride, any row pitch): NaN / Inf guards,
+    z = logits / temperature, the top-p nucleus (tokens whose strictly-larger-z mass is < top_p), then the
+    Gumbel-max draw keyed by Philox4x32-10 of (seed, row, step); the rule is stated in b200_bridge.h.
+    `seed` is a one-element int64 CUDA tensor read when the kernel runs. Returns `out` (int64 [rows], any
+    stride; allocated when None)."""
+    _need_cuda(logits, seed, out)
+    if logits.dim() != 2 or logits.stride(1) != 1:
+        raise RuntimeError("sample_tokens: logits must be 2-D with unit inner stride")
+    if logits.dtype not in (torch.float32, torch.bfloat16):
+        raise RuntimeError("sample_tokens: logits must be fp32 or bf16")
+    if seed.dtype != torch.int64 or seed.numel() != 1:
+        raise RuntimeError("sample_tokens: seed must be a one-element int64 tensor")
+    rows, vocab = logits.shape
+    if out is None:
+        out = torch.empty(rows, device=logits.device, dtype=torch.int64)
+    if out.dtype != torch.int64 or out.dim() != 1 or out.shape[0] != rows:
+        raise RuntimeError("sample_tokens: `out` must be int64 [rows]")
+    ld = logits.stride(0) if rows > 1 else max(logits.stride(0), vocab)
+    _lib.check(_lib.lib().b200b_sample_tokens(logits.data_ptr(), 1 if logits.dtype == torch.bfloat16 else 0, ld, rows,
+                                              vocab, float(temperature), float(top_p), seed.data_ptr(), int(step),
+                                              out.data_ptr(), out.stride(0), _stream_ptr()), "sample_tokens")
+    return out
+
+
 def gemm_grad_pair(dy: torch.Tensor, w: torch.Tensor, x: torch.Tensor, *, wgrad_dtype: torch.dtype = torch.float32):
     """dX = dY W (bf16 [rows, n_in]) and dW = dY^T X ([n_out, n_in], fp32 or bf16) of one Linear through
     b200b_gemm_dual: ONE grouped persistent launch when both fit 256 x 128 pair tiles, two launches otherwise.
