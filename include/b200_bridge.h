@@ -480,6 +480,89 @@ int b200b_sample_tokens(const void* logits, int dtype, int64_t ld, int64_t rows,
                         float top_p, const unsigned long long* seed, int64_t step, int64_t* ids_out,
                         int64_t ids_stride, void* stream);
 
+/* ------------------------------------------------------------------------------------------- *
+ * Beam search, one step for `batch` images of K beams each (csrc/beam.cu). Replaces the per-step scoring and
+ * selection of Hugging Face generate(num_beams=K) (log_softmax, add the beam scores, top-2K over K * V,
+ * BeamHypotheses.add / is_done), which the reference can only run as a loop over replicated images.
+ *
+ * The rule, per image b with K beams (1 <= K <= 8), EOS id eos (-1: none), length penalty alpha (finite) and
+ * early_stopping in {0, 1}:
+ *  state: K running beams (a prefix of ids and a log-probability sum s_k each), a finished set of at most K
+ *         hypotheses (normalised score, ids, length) and a done flag. Start: every beam holds [BOS], s_0 = 0,
+ *         s_k = -inf for k > 0 (the first step expands beam 0 only), the finished set is empty.
+ *  step t writes position t + 1; n = t + 1 counts the generated tokens after it, INCLUDING an EOS (Hugging Face
+ *  versions differ on this; here the EOS counts):
+ *   1. the NaN / Inf guards of the greedy path on each beam's logit row: a row with a NaN becomes all zeros;
+ *      otherwise a row with an Inf is clamped to [-100, 100];
+ *   2. lse_k = log sum_v exp(z_kv) in fp32; candidate score c_kv = fl(s_k + fl(z_kv - lse_k));
+ *   3. order the K * V candidates by c descending, ties by z descending, then by the smaller flat index
+ *      k * V + v; keep the first 2K. NOTE this is not a tie-break by flat index alone: two candidates with equal
+ *      c and different z (e.g. of two beams) go by z, not by index. The reason: c is non-decreasing in z within
+ *      a beam, and with the z tie-break the first 2K are always among each beam's 2K largest z (smaller v first),
+ *      also where two z of one beam round to the same c -- so each row only needs its 2K best z. With a tie-break
+ *      by index alone, such a rounding tie could select a candidate outside its row's 2K best z. Equal c with
+ *      equal z (duplicates) still go by flat index. A NaN c (only from a NaN the caller put in beam_scores)
+ *      counts as -inf.
+ *   4. walk the kept candidates in order: an EOS candidate at rank r < K is offered to the finished set with
+ *      score c / N (N below); an EOS candidate at rank r >= K is skipped; any other candidate becomes the next
+ *      beam (parent k, token v, score c) until K beams are chosen. The finished set keeps its K best: a newcomer
+ *      is added while it holds fewer than K, and otherwise evicts the worst entry (ties: the one added first)
+ *      only if its score is strictly greater;
+ *   5. done: early_stopping = 1: once the finished set holds K entries; early_stopping = 0 (the Hugging Face
+ *      heuristic): once it holds K entries and its worst score is >= max_k s'_k / N over the new beams.
+ *      A done image is frozen: later steps leave its beams, scores and finished set bit-for-bit unchanged (its
+ *      rows still flow through the bridge; its ids rows are copied unchanged and position t + 1 gets
+ *      max(eos, 0), so the next embedding lookup stays in range; its parents are the identity).
+ *  N = powf(n, alpha) in fp32, clamped to [FLT_MIN, FLT_MAX] (so no score is NaN for any finite alpha).
+ *  after the last step (b200b_beam_finalize, n = steps): for each image that is not done, running beams
+ *  k = 0..K-1 are offered in that order with score s_k / N and length n; the result is the finished hypothesis
+ *  with the best score, ties to the one added first. A hypothesis that ended in EOS at step t has caption length
+ *  t + 1 (BOS + t tokens; the EOS at position t + 1 is not part of it).
+ *  V >= 2 is required, so the first 2K always hold at least K candidates that are not EOS.
+ *
+ * State (caller-owned device buffers, R = batch * K rows, beam k of image b is row b * K + k). Initialise
+ * beam_scores to 0 at k = 0 and -inf elsewhere, hyp_count and done to 0; the other fields need no initial value.
+ * Whatever the state holds, every index the kernels derive from it stays in range (a negative hyp_count counts as 0).
+ * b200b_beam_step reads and updates it; b200b_beam_finalize only reads it.
+ * ------------------------------------------------------------------------------------------- */
+typedef struct b200b_beam_state {
+  float* beam_scores;  /* [R]  s_k of the running beams                                         */
+  float* hyp_scores;   /* [R]  finished set of image b: slots b*K .. b*K+K-1, normalised scores  */
+  int32_t* hyp_lens;   /* [R]  caption length + 1 (BOS and the tokens, EOS excluded)             */
+  int32_t* hyp_seq;    /* [R]  order in which the slot's hypothesis was added (ties)             */
+  int32_t* hyp_count;  /* [batch] hypotheses accepted so far (filled slots = min(count, K))     */
+  int32_t* done;       /* [batch] 0 / 1                                                          */
+  int64_t* hyp_ids;    /* [R][ld_hyp] ids of each finished hypothesis: BOS, tokens, EOS          */
+  int64_t ld_hyp;
+} b200b_beam_state;
+
+/* One step t = `step` of the rule above. logits [R, vocab] (row pitch ld >= vocab, dtype 0 = f32, 1 = bf16,
+ * nothing beyond vocab is read); ids int64 [R][ld_ids] holds every beam's prefix at positions 0..t; the step
+ * writes the new beams to ids_next (another buffer, same pitch): ids_next[b*K + k, 0..t] = ids[b*K + parent,
+ * 0..t], ids_next[b*K + k, t + 1] = token; parents int64 [R] receives b*K + parent (a row of the same image,
+ * for reordering per-beam caches); a hypothesis that finishes is copied to hyp_ids with its EOS. Two launches:
+ * a per-row pass that reads each logit row from HBM once (running max, sum of exp, NaN / Inf flags and the
+ * row's 2K best z; a row split over a cluster of CTAs as in b200b_sample_tokens; only rows with a NaN or Inf
+ * take a second, guarded pass) and one CTA per image for steps 3-5.
+ * B200B_ERR_ARG: a null pointer, ids == ids_next, dtype not 0 / 1, K outside [1, 8], eos outside [-1, vocab),
+ * ld < vocab, ld_ids or ld_hyp < step + 2, step < 0, alpha not finite, early_stopping not 0 / 1.
+ * B200B_ERR_SHAPE: batch < 1, vocab < 2, vocab above the sampler's limit (360448 f32 / 720896 bf16), R * 8
+ * or K * vocab above 2^31 - 1. B200B_ERR_WORKSPACE: workspace_bytes < b200b_beam_step_workspace_bytes(batch, K)
+ * (0 for bad arguments). */
+size_t b200b_beam_step_workspace_bytes(int64_t batch, int num_beams);
+int b200b_beam_step(const void* logits, int dtype, int64_t ld, int64_t batch, int num_beams, int64_t vocab,
+                    int64_t eos, float length_penalty, int early_stopping, int64_t step, const int64_t* ids,
+                    int64_t* ids_next, int64_t ld_ids, int64_t* parents, const b200b_beam_state* state,
+                    void* workspace, size_t workspace_bytes, void* stream);
+/* The "after the last step" rule for `steps` >= 1 steps, without changing the state. ids [R][ld_ids] holds the
+ * running beams (positions 0..steps). out_ids int64 [batch][ld_out]: positions 0..steps of the result, with
+ * max(eos, 0) after its length; out_len int64 [batch]: its caption length + 1 (ids[b, 1:out_len[b]] is the
+ * caption); out_score f32 [batch]: its normalised score. B200B_ERR_ARG: a null pointer, K outside [1, 8],
+ * eos < -1, ld_ids, ld_hyp or ld_out < steps + 1, alpha not finite; B200B_ERR_SHAPE: batch < 1, steps < 1. */
+int b200b_beam_finalize(int64_t batch, int num_beams, int64_t eos, float length_penalty, int64_t steps,
+                        const int64_t* ids, int64_t ld_ids, const b200b_beam_state* state, int64_t* out_ids,
+                        int64_t ld_out, int64_t* out_len, float* out_score, void* stream);
+
 /* out f32 [n] = scale * in bf16 [n] (n % 8 == 0): turns an exchanged bf16 gradient bucket into
  * the fp32 .grad the optimizer reads. */
 int b200b_bf16_to_f32(const void* in_bf16, float* out, int64_t n, float scale, void* stream);

@@ -62,6 +62,13 @@ class NvlsComm(C.Structure):
                 ("error_word", C.c_void_p)]
 
 
+class BeamState(C.Structure):
+    """b200b_beam_state"""
+    _fields_ = [("beam_scores", C.c_void_p), ("hyp_scores", C.c_void_p), ("hyp_lens", C.c_void_p),
+                ("hyp_seq", C.c_void_p), ("hyp_count", C.c_void_p), ("done", C.c_void_p), ("hyp_ids", C.c_void_p),
+                ("ld_hyp", C.c_int64)]
+
+
 class AttnArgs(C.Structure):
     _fields_ = [
         ("q", C.c_void_p), ("ldq", C.c_int64),
@@ -148,6 +155,16 @@ def _declare(lib) -> None:
     lib.b200b_sample_tokens.restype = C.c_int
     lib.b200b_sample_tokens.argtypes = [C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_int64, C.c_float, C.c_float,
                                         C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]
+    lib.b200b_beam_step_workspace_bytes.restype = C.c_size_t
+    lib.b200b_beam_step_workspace_bytes.argtypes = [C.c_int64, C.c_int]
+    lib.b200b_beam_step.restype = C.c_int
+    lib.b200b_beam_step.argtypes = [C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_int, C.c_int64, C.c_int64, C.c_float,
+                                    C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p,
+                                    C.POINTER(BeamState), C.c_void_p, C.c_size_t, C.c_void_p]
+    lib.b200b_beam_finalize.restype = C.c_int
+    lib.b200b_beam_finalize.argtypes = [C.c_int64, C.c_int, C.c_int64, C.c_float, C.c_int64, C.c_void_p, C.c_int64,
+                                        C.POINTER(BeamState), C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
+                                        C.c_void_p]
     lib.b200b_gemm_dual.restype = C.c_int
     lib.b200b_gemm_dual.argtypes = [C.POINTER(GemmArgs), C.POINTER(GemmArgs), C.c_void_p]
     lib.b200b_gemm_set_dual.restype = C.c_int

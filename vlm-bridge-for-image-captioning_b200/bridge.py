@@ -576,6 +576,10 @@ class BridgeLite(nn.Module):
 
     def _run_forward(self, vision: torch.Tensor, text: torch.Tensor, keep_for_backward: bool, kv_cache=None,
                      block_callback=None, cached_positions: Optional[int] = None):
+        if kv_cache is not None and getattr(kv_cache, "beams", 1) > 1:
+            if keep_for_backward:
+                raise RuntimeError("a beam-search cache is inference-only")
+            return self._run_forward_beams(text, kv_cache, block_callback, cached_positions), None
         self._ensure_flat()
         self._refresh_bf16()
         dev = self._flat.device
@@ -660,6 +664,8 @@ class BridgeLite(nn.Module):
         """Inference forward with fp32 operands over an fp32 `VisionKVCache` (csrc/exact_fp32.cu): the
         reference's decode numerics (no autocast, full_model.py:221-261). Same block / position-row
         structure as `_run_forward`."""
+        if getattr(kv_cache, "beams", 1) > 1:
+            return self._run_forward_beams(text, kv_cache, block_callback, cached_positions)
         self._ensure_flat()
         dev = self._flat.device
         if self.training and self.dropout_p > 0:
@@ -675,12 +681,7 @@ class BridgeLite(nn.Module):
         dims = self._dims(B, L, Nv)
         ws_bytes = lib.b200b_bridge_f32_workspace_bytes(C.byref(dims))
         ws = torch.empty(ws_bytes, device=dev, dtype=torch.uint8)
-        b32 = self._flat.data_ptr()
-        ptrs = self.__dict__.get("_ptrs32")
-        if ptrs is None or ptrs[0] != b32:
-            ptrs = (b32, [self._block_ptr_struct(0, b32, i, grads=False) for i in range(self.num_blocks)])
-            self.__dict__["_ptrs32"] = ptrs
-        ptrs = ptrs[1]
+        ptrs = self._f32_ptrs()
         st = _stream()
         kv = kv_cache.kv32
         pos_cache = None
@@ -709,6 +710,87 @@ class BridgeLite(nn.Module):
                 block_callback(i, cur.view(B, L, D), x_out.view(B, L, D))
             cur = x_out
         return cur.view(B, L, D)
+
+    def _f32_ptrs(self):
+        """Block pointer structs of the fp32 path (every field in the fp32 arena), cached per arena address."""
+        b32 = self._flat.data_ptr()
+        ptrs = self.__dict__.get("_ptrs32")
+        if ptrs is None or ptrs[0] != b32:
+            ptrs = (b32, [self._block_ptr_struct(0, b32, i, grads=False) for i in range(self.num_blocks)])
+            self.__dict__["_ptrs32"] = ptrs
+        return ptrs[1]
+
+    def _run_forward_beams(self, text: torch.Tensor, kv_cache, block_callback=None,
+                           cached_positions: Optional[int] = None) -> torch.Tensor:
+        """Inference forward over a beam-search cache (`VisionKVCache(..., beams=K)`, either precision): text
+        [B*K, L, D], rows [B][K][L], over the K/V of B images. Every block runs as two calls on the same buffers:
+        the cross-attention sub-layer with dims (batch=B, len_text=K*L) -- image b's K*L rows are one query block
+        over its cache, which is read once for all its beams -- and the rest of the block with dims
+        (batch=B*K, len_text=L), so that the self-attention and the FFN stay within a beam. Both dims come from
+        the cache's (batch, beams), after the text batch is checked against them."""
+        B, K = int(kv_cache.batch), int(kv_cache.beams)
+        if text.dim() != 3 or int(text.shape[0]) != B * K:
+            raise RuntimeError(f"a cache of {B} images x {K} beams needs text_embeddings [{B * K}, L, "
+                               f"{self.language_dim}], got {tuple(text.shape)}")
+        self._ensure_flat()
+        fp32 = kv_cache.precision == "fp32"
+        if self.training and self.dropout_p > 0:
+            raise RuntimeError("a beam-search cache needs inference mode: call .eval() first")
+        if not fp32:
+            self._refresh_bf16()
+        dev = self._flat.device
+        if text.device != dev or text.shape[-1] != self.language_dim:
+            raise RuntimeError(f"text_embeddings must be a CUDA tensor [B*K, L, {self.language_dim}] on the module's device")
+        x = text.detach().to(torch.float32).contiguous()
+        _, L, D = x.shape
+        Nv = kv_cache.len_vision
+        lib = _bridge_lib()
+        st = _stream()
+        pos_cache, k0 = None, 0
+        if cached_positions is not None:
+            pos_cache = kv_cache.position_rows(L, cached_positions, dev, D)
+            k0 = int(cached_positions) if pos_cache is not None else 0
+        rdims = self._dims(B * K, L, Nv, FLAG_PART_REST)
+        full_cross = self._dims(B, K * L, Nv, FLAG_PART_CROSS)
+        if fp32:
+            ptrs, kv = self._f32_ptrs(), kv_cache.kv32
+            ws_bytes = max(lib.b200b_bridge_f32_workspace_bytes(C.byref(d)) for d in (rdims, full_cross))
+        else:
+            ptrs, kv = self._weight_ptrs(), kv_cache.kv
+            ws_bytes = max(lib.b200b_bridge_block_saved_bytes(C.byref(d)) for d in (rdims, full_cross))
+        ws = torch.empty(ws_bytes, device=dev, dtype=torch.uint8)
+
+        def block(dims, i, x_in, kv_t, x_out, what):
+            if fp32:
+                rc = lib.b200b_bridge_block_forward_f32(C.byref(dims), i, C.byref(ptrs[i]), x_in.data_ptr(), kv_t.data_ptr(),
+                                                        x_out.data_ptr(), ws.data_ptr(), ws_bytes, st)
+            else:
+                rc = lib.b200b_bridge_block_forward(C.byref(dims), i, C.byref(ptrs[i]), x_in.data_ptr(), kv_t.data_ptr(),
+                                                    x_out.data_ptr(), ws.data_ptr(), ws_bytes, 0.0, 0, st)
+            _lib.check(rc, what)
+
+        def cross(i, x_in, n):
+            """x1 [B*K*n, D] of the cross-attention sub-layer for n positions of every beam"""
+            kv_t, flag = (kv, 0) if fp32 else self._kv_flag(kv_cache, K * n, False)
+            x1 = torch.empty((B * K * n, D), device=dev, dtype=torch.float32)
+            block(self._dims(B, K * n, Nv, flag | FLAG_PART_CROSS), i, x_in, kv_t, x1, "block_forward(beams, cross part)")
+            return x1
+
+        cur = x.view(B * K * L, D)
+        for i in range(self.num_blocks):
+            if i == 0 and pos_cache is not None:
+                n_new = L - k0
+                x1_new = cross(0, x[:, k0:, :].contiguous(), n_new)
+                pos_cache[:, k0:L].copy_(x1_new.view(B * K, n_new, D))
+                x1 = pos_cache[:, :L].contiguous().view(B * K * L, D)
+            else:
+                x1 = cross(i, cur, L)
+            x_out = torch.empty((B * K * L, D), device=dev, dtype=torch.float32)
+            block(rdims, i, x1, kv, x_out, "block_forward(beams, rest)")
+            if block_callback is not None:
+                block_callback(i, cur.view(B * K, L, D), x_out.view(B * K, L, D))
+            cur = x_out
+        return cur.view(B * K, L, D)
 
     def _run_backward(self, state, d_out: torch.Tensor, text_needs_grad: bool):
         lay = self._layout

@@ -24,6 +24,11 @@ int device_sm_count(int* out);
 int make_tmap_heads_sw64(CUtensorMap* tm, const void* base, long long ld_elems, int head_dim, int heads, int rows,
                          int batch, int box_rows);
 
+// How many CTAs (1, 2, 4 or 8; 0 if the row is too long) one vocabulary row of `vocab` elements of `esz` bytes is
+// split over when `rows` rows run on `sms` SMs, and each CTA's slice (`*slice` tokens, a multiple of 8). Shared by
+// the sampler (csrc/sampling.cu) and the beam step (csrc/beam.cu).
+int sample_cluster_size(long long rows, long long vocab, int esz, int sms, long long* slice);
+
 // Which kernel families are launched with programmatic stream serialization: bit mask from the
 // environment variable B200B_PDL (1 = GEMMs, 2 = attention, 4 = row / column / cast kernels).
 enum { kPdlGemm = 1, kPdlAttn = 2, kPdlRows = 4 };

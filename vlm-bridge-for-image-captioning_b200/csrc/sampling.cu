@@ -336,7 +336,8 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(kSampThreads, 1)
 
 // Cluster size: the fewest CTAs whose slices fit kSampSliceBytes, doubled (up to kSampMaxCluster) while the
 // rows * CTAs do not cover the SMs and every CTA keeps at least 4096 tokens. 0 if the row does not fit.
-static int sample_cluster_size(long long rows, long long vocab, int esz, int sms, long long* slice) {
+// The beam-step kernel (csrc/beam.cu) splits its rows by the same rule.
+int sample_cluster_size(long long rows, long long vocab, int esz, int sms, long long* slice) {
   auto slice_of = [&](int c) { return ((vocab + c - 1) / c + 7) / 8 * 8; };
   int c = 1;
   while (c <= kSampMaxCluster && slice_of(c) * esz > kSampSliceBytes) c *= 2;

@@ -29,7 +29,7 @@ import torch
 from . import ops
 from .kv_cache import VisionKVCache
 
-__all__ = ["greedy_decode", "DecodeStepGraphs"]
+__all__ = ["greedy_decode", "beam_search_decode", "DecodeStepGraphs"]
 
 
 class DecodeStepGraphs:
@@ -77,6 +77,31 @@ class DecodeStepGraphs:
         static_in.copy_(text_embeddings, non_blocking=True)
         g.replay()
         return out
+
+
+def _decode_setup(bridge, vision_features, max_new_tokens, kv_cache, use_cache, step_graphs, use_graphs, precision,
+                  refill_cache, beams: int = 1):
+    """The argument, cache and graph setup of the decode drivers: (kv_cache, step_graphs) to use."""
+    if precision not in ("bf16", "fp32"):
+        raise ValueError("precision must be 'bf16' or 'fp32'")
+    if precision == "fp32" and not use_cache:
+        raise RuntimeError("precision='fp32' reads an fp32 VisionKVCache: use_cache must stay True")
+    if kv_cache is not None and use_cache and getattr(kv_cache, "beams", 1) != beams:
+        raise ValueError(f"kv_cache was built for beams={kv_cache.beams}, this decode runs {beams}")
+    if use_cache and kv_cache is None:
+        kv_cache = VisionKVCache(bridge, vision_features, precision=precision, max_positions=max(64, max_new_tokens),
+                                 beams=beams)
+    elif use_cache:
+        if kv_cache.precision != precision:
+            raise RuntimeError(f"kv_cache holds {kv_cache.precision} K/V but precision={precision!r} was asked for")
+        if refill_cache:
+            kv_cache.refill(vision_features)
+    if (use_graphs or step_graphs is not None) and use_cache:
+        if step_graphs is None or step_graphs.cache is not kv_cache:
+            step_graphs = DecodeStepGraphs(bridge, kv_cache)
+    else:
+        step_graphs = None
+    return kv_cache, step_graphs
 
 
 @torch.no_grad()
@@ -129,23 +154,8 @@ def greedy_decode(bridge, vision_features: torch.Tensor, embed_fn: Callable[[tor
                 gdev = torch.device("cuda", torch.cuda.current_device())
             if gdev is not None and gdev != dev:
                 raise ValueError(f"generator is on {generator.device}, the images on {dev}")
-        if precision not in ("bf16", "fp32"):
-            raise ValueError("precision must be 'bf16' or 'fp32'")
-        if precision == "fp32" and not use_cache:
-            raise RuntimeError("precision='fp32' reads an fp32 VisionKVCache: use_cache must stay True")
-        if use_cache and kv_cache is None:
-            kv_cache = VisionKVCache(bridge, vision_features, precision=precision,
-                                     max_positions=max(64, max_new_tokens))
-        elif use_cache:
-            if kv_cache.precision != precision:
-                raise RuntimeError(f"kv_cache holds {kv_cache.precision} K/V but precision={precision!r} was asked for")
-            if refill_cache:
-                kv_cache.refill(vision_features)
-        if (use_graphs or step_graphs is not None) and use_cache:
-            if step_graphs is None or step_graphs.cache is not kv_cache:
-                step_graphs = DecodeStepGraphs(bridge, kv_cache)
-        else:
-            step_graphs = None
+        kv_cache, step_graphs = _decode_setup(bridge, vision_features, max_new_tokens, kv_cache, use_cache, step_graphs,
+                                              use_graphs, precision, refill_cache)
         ids = torch.empty((B, 1 + max_new_tokens), dtype=torch.long, device=dev)
         ids[:, 0] = bos_token_id
         if do_sample:
@@ -181,5 +191,68 @@ def greedy_decode(bridge, vision_features: torch.Tensor, embed_fn: Callable[[tor
             first = torch.where(is_eos.any(dim=1), is_eos.float().argmax(dim=1), torch.full((B,), max_new_tokens, device=dev))
             lengths = first + 1
         return ids, lengths
+    finally:
+        bridge.train(was_training)
+
+
+@torch.no_grad()
+def beam_search_decode(bridge, vision_features: torch.Tensor, embed_fn: Callable[[torch.Tensor], torch.Tensor],
+                       lm_fn: Callable[[torch.Tensor], torch.Tensor], *, num_beams: int, bos_token_id: int,
+                       eos_token_id: Optional[int] = None, max_new_tokens: int = 50, length_penalty: float = 1.0,
+                       early_stopping: bool = False, kv_cache: Optional[VisionKVCache] = None,
+                       step_graphs: Optional[DecodeStepGraphs] = None, use_graphs: bool = False,
+                       precision: str = "bf16", refill_cache: bool = False):
+    """Beam search over B images with `num_beams` = K beams each (generate(num_beams=K) of the Hugging Face stack the
+    language model comes from; the rule, including where it differs from Hugging Face, is stated in
+    include/b200_bridge.h at b200b_beam_step). Returns (ids [B, 1 + max_new_tokens] int64 incl. BOS, lengths [B]
+    int64, scores [B] fp32): image b's caption is ids[b, 1:lengths[b]] (EOS excluded, as in `greedy_decode`) and
+    scores[b] its sum of log-probabilities divided by n ** length_penalty.
+
+    The B*K beam rows share their image's K/V (`VisionKVCache(..., beams=K)`): the cross-attention reads each
+    image's cache once for all its beams. `embed_fn` / `lm_fn` see B*K rows, [B][K] (as in `greedy_decode`).
+    Each step runs the bridge on the beams' prefixes, then one fused beam step on the logits of their last
+    positions (`ops.beam_step`: log-softmax, scores, top-2K, finished hypotheses, the new beams' ids), then
+    reorders the cached position rows by the chosen parents; nothing waits for the host, eagerly or with step
+    graphs (`use_graphs` / `step_graphs`, as in `greedy_decode`). All beams run `max_new_tokens` steps in lock-step:
+    an image whose search is done keeps its result while its rows keep flowing through the bridge.
+    `num_beams` outside [1, 8], a non-finite `length_penalty`, a `kv_cache` built for another number of beams or a
+    `precision` other than "bf16" / "fp32" raise ValueError before any kernel runs."""
+    K = int(num_beams)
+    if not 1 <= K <= 8:
+        raise ValueError(f"num_beams must be in [1, 8], got {num_beams}")
+    length_penalty = float(length_penalty)
+    if not math.isfinite(length_penalty):
+        raise ValueError(f"length_penalty must be finite, got {length_penalty}")
+    if int(max_new_tokens) < 1:
+        raise ValueError(f"max_new_tokens must be >= 1, got {max_new_tokens}")
+    was_training = bridge.training
+    bridge.eval()
+    try:
+        kv_cache, step_graphs = _decode_setup(bridge, vision_features, max_new_tokens, kv_cache, True, step_graphs,
+                                              use_graphs, precision, refill_cache, beams=K)
+        B = vision_features.shape[0]
+        dev = vision_features.device
+        T = int(max_new_tokens)
+        ids = torch.empty((B * K, 1 + T), dtype=torch.long, device=dev)
+        ids[:, 0] = bos_token_id
+        ids_next = torch.empty_like(ids)
+        parents = torch.empty(B * K, dtype=torch.long, device=dev)
+        state = ops.BeamState(B, K, 1 + T, dev)
+        for step in range(T):
+            prefix = ids[:, :step + 1]
+            if step_graphs is not None:
+                hidden = step_graphs(embed_fn(prefix), cached_positions=step)
+            else:
+                hidden = bridge(vision_features, embed_fn(prefix), kv_cache=kv_cache, cached_positions=step)
+            logits = lm_fn(hidden)
+            if logits.dim() == 3:
+                logits = logits[:, -1, :]
+            if logits.dtype not in (torch.float32, torch.bfloat16) or logits.stride(-1) != 1:
+                logits = logits.float().contiguous()
+            ops.beam_step(logits, ids, ids_next, parents, state, step=step, eos_token_id=eos_token_id,
+                          length_penalty=length_penalty, early_stopping=early_stopping)
+            kv_cache.reorder_beams(parents)
+            ids, ids_next = ids_next, ids
+        return ops.beam_finalize(ids, state, steps=T, eos_token_id=eos_token_id, length_penalty=length_penalty)
     finally:
         bridge.train(was_training)

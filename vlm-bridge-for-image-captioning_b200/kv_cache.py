@@ -19,6 +19,11 @@ which involves no other text position, so a decode loop that appends tokens comp
 position (`BridgeLite.forward(..., kv_cache=cache, cached_positions=k)`) instead of once per position
 per step. Everything after it (block 0's non-causal self-attention onwards) mixes positions and is
 recomputed on the whole prefix, as in the reference.
+
+Beam search (`beams=K`): the K beams of an image attend to the same image K/V, so the K/V buffers stay per image
+(B images) and only the position rows grow to one per beam (`x1` [B*K, max_positions, D], row b*K + k).
+`BridgeLite` runs the cross-attention of the B*K text rows as B query blocks of K*s rows over the image's cache and
+the rest of each block per beam; `reorder_beams(parents)` follows the beams chosen by a step.
 """
 from __future__ import annotations
 
@@ -33,12 +38,16 @@ class VisionKVCache:
     inference path (csrc/exact_fp32.cu) -- the numerics of the reference's own decode, which runs without
     autocast (full_model.py:221-261); greedy token ids then equal the fp32 reference's on every step."""
 
-    def __init__(self, bridge, vision_features: torch.Tensor, max_positions: int = 64, precision: str = "bf16"):
+    def __init__(self, bridge, vision_features: torch.Tensor, max_positions: int = 64, precision: str = "bf16",
+                 beams: int = 1):
         if vision_features.dim() != 3:
             raise RuntimeError("vision_features must be [B, Nv, vision_dim]")
         if precision not in ("bf16", "fp32"):
             raise ValueError("precision must be 'bf16' or 'fp32'")
+        if not 1 <= int(beams) <= 8:
+            raise ValueError(f"beams must be in [1, 8], got {beams}")
         self.precision = precision
+        self.beams = int(beams)
         self._bridge = bridge
         self.max_positions = int(max_positions)
         self.batch, self.len_vision = int(vision_features.shape[0]), int(vision_features.shape[1])
@@ -64,7 +73,8 @@ class VisionKVCache:
         self._versions = tuple(p._version for p in bridge.parameters())
         dev = self.kv32.device if self.precision == "fp32" else self.kv.device
         if self.x1 is None and self.max_positions > 0:
-            self.x1 = torch.empty((self.batch, self.max_positions, bridge.language_dim), device=dev, dtype=torch.float32)
+            self.x1 = torch.empty((self.batch * self.beams, self.max_positions, bridge.language_dim), device=dev,
+                                  dtype=torch.float32)
         self.positions_filled = 0
         return self
 
@@ -99,6 +109,17 @@ class VisionKVCache:
             raise RuntimeError("position rows live on another device / have another width than the text")
         self.positions_filled = length
         return self.x1
+
+    def reorder_beams(self, parents: torch.Tensor) -> None:
+        """Beam search: position-row store row r takes the filled rows of row parents[r], in place (the buffer
+        keeps its address, so captured graphs stay valid). `parents` int64 [batch * beams] is what
+        `ops.beam_step` wrote: b * beams + (a beam of image b), in range by construction."""
+        if parents.dtype != torch.int64 or parents.shape != (self.batch * self.beams,):
+            raise RuntimeError(f"parents must be int64 [{self.batch * self.beams}]")
+        if self.x1 is None or self.positions_filled == 0:
+            return
+        rows = self.x1[:, :self.positions_filled]
+        rows.copy_(rows.index_select(0, parents))
 
     @property
     def nbytes(self) -> int:

@@ -305,6 +305,105 @@ def sample_tokens(logits: torch.Tensor, *, temperature: float, top_p: float, see
     return out
 
 
+def _same_device(what: str, *ts: torch.Tensor) -> None:
+    if any(t.device != ts[0].device for t in ts[1:]):
+        raise RuntimeError(f"{what}: every tensor and the beam state must be on one device")
+
+
+class BeamState:
+    """Device state of a beam search over `batch` images x `num_beams` beams with room for `max_len` positions
+    (b200b_beam_state: running scores, the finished set of each image, done flags) plus the step workspace. Rows
+    are [batch][num_beams]. `reset()` restores the start state (s_0 = 0, s_k = -inf, empty finished sets) with
+    device fills only, so a decode loop or a captured graph can reuse the buffers."""
+
+    def __init__(self, batch: int, num_beams: int, max_len: int, device):
+        if not 1 <= int(num_beams) <= 8:
+            raise ValueError(f"num_beams must be in [1, 8], got {num_beams}")
+        self.batch, self.num_beams, self.max_len = int(batch), int(num_beams), int(max_len)
+        R = self.batch * self.num_beams
+        self.beam_scores = torch.empty(R, device=device, dtype=torch.float32)
+        self.hyp_scores = torch.empty(R, device=device, dtype=torch.float32)
+        self.hyp_lens = torch.empty(R, device=device, dtype=torch.int32)
+        self.hyp_seq = torch.empty(R, device=device, dtype=torch.int32)
+        self.hyp_count = torch.empty(self.batch, device=device, dtype=torch.int32)
+        self.done = torch.empty(self.batch, device=device, dtype=torch.int32)
+        self.hyp_ids = torch.empty((R, self.max_len), device=device, dtype=torch.int64)
+        nbytes = _lib.lib().b200b_beam_step_workspace_bytes(self.batch, self.num_beams)
+        if nbytes == 0:
+            raise RuntimeError("beam_step_workspace_bytes: bad batch / num_beams")
+        self.workspace = torch.empty(nbytes, device=device, dtype=torch.uint8)
+        self.struct = _lib.BeamState(self.beam_scores.data_ptr(), self.hyp_scores.data_ptr(), self.hyp_lens.data_ptr(),
+                                     self.hyp_seq.data_ptr(), self.hyp_count.data_ptr(), self.done.data_ptr(),
+                                     self.hyp_ids.data_ptr(), self.max_len)
+        self.reset()
+
+    def reset(self) -> "BeamState":
+        self.beam_scores.view(self.batch, self.num_beams).fill_(-float("inf"))[:, 0] = 0.0
+        self.hyp_scores.fill_(-float("inf"))
+        self.hyp_count.zero_()
+        self.done.zero_()
+        return self
+
+
+def beam_step(logits: torch.Tensor, ids: torch.Tensor, ids_next: torch.Tensor, parents: torch.Tensor,
+              state: BeamState, *, step: int, eos_token_id: int | None, length_penalty: float = 1.0,
+              early_stopping: bool = False) -> None:
+    """One beam-search step (b200b_beam_step; the rule is stated in b200_bridge.h). logits [batch * K, V] (fp32 or
+    bf16, unit inner stride, any row pitch) of the beams' last positions; ids / ids_next int64 [batch * K, >= step + 2]
+    (contiguous rows, same pitch): the step reads positions 0..step of ids and writes positions 0..step + 1 of the
+    new beams to ids_next; parents int64 [batch * K] receives each new beam's parent row (b * K + parent)."""
+    _need_cuda(logits, ids, ids_next, parents)
+    if logits.dim() != 2 or logits.stride(1) != 1:
+        raise RuntimeError("beam_step: logits must be 2-D with unit inner stride")
+    if logits.dtype not in (torch.float32, torch.bfloat16):
+        raise RuntimeError("beam_step: logits must be fp32 or bf16")
+    R = state.batch * state.num_beams
+    rows, vocab = logits.shape
+    if rows != R:
+        raise RuntimeError(f"beam_step: logits have {rows} rows, the state {state.batch} x {state.num_beams}")
+    for name, t in (("ids", ids), ("ids_next", ids_next)):
+        if t.dtype != torch.int64 or t.dim() != 2 or t.shape[0] != R or t.stride(1) != 1:
+            raise RuntimeError(f"beam_step: {name} must be int64 [batch * K, L] with unit inner stride")
+    if ids.stride(0) != ids_next.stride(0):
+        raise RuntimeError("beam_step: ids and ids_next must have the same row pitch")
+    if parents.dtype != torch.int64 or parents.shape != (R,) or not parents.is_contiguous():
+        raise RuntimeError("beam_step: parents must be a contiguous int64 [batch * K]")
+    if ids.shape[1] < int(step) + 2 or ids_next.shape[1] < int(step) + 2:
+        raise RuntimeError(f"beam_step: ids and ids_next need >= step + 2 = {int(step) + 2} columns (step {step} writes "
+                           "position step + 1)")
+    _same_device("beam_step", logits, ids, ids_next, parents, state.beam_scores)
+    ld = logits.stride(0) if rows > 1 else max(logits.stride(0), vocab)
+    eos = -1 if eos_token_id is None else int(eos_token_id)
+    _lib.check(_lib.lib().b200b_beam_step(
+        logits.data_ptr(), 1 if logits.dtype == torch.bfloat16 else 0, ld, state.batch, state.num_beams, vocab, eos,
+        float(length_penalty), 1 if early_stopping else 0, int(step), ids.data_ptr(), ids_next.data_ptr(),
+        ids.stride(0), parents.data_ptr(), C.byref(state.struct), state.workspace.data_ptr(),
+        state.workspace.numel(), _stream_ptr()), "beam_step")
+
+
+def beam_finalize(ids: torch.Tensor, state: BeamState, *, steps: int, eos_token_id: int | None,
+                  length_penalty: float = 1.0):
+    """The "after the last step" rule of b200b_beam_finalize over the running beams ids [batch * K, >= steps + 1]
+    after `steps` steps; the state is not changed. Returns (ids int64 [batch, 1 + steps], lengths int64 [batch],
+    scores fp32 [batch]): ids[b, 1:lengths[b]] is image b's caption, EOS excluded."""
+    _need_cuda(ids)
+    R = state.batch * state.num_beams
+    if ids.dtype != torch.int64 or ids.dim() != 2 or ids.shape[0] != R or ids.stride(1) != 1:
+        raise RuntimeError("beam_finalize: ids must be int64 [batch * K, L] with unit inner stride")
+    if ids.shape[1] < int(steps) + 1:
+        raise RuntimeError(f"beam_finalize: ids need >= steps + 1 = {int(steps) + 1} columns")
+    _same_device("beam_finalize", ids, state.beam_scores)
+    out = torch.empty((state.batch, 1 + int(steps)), device=ids.device, dtype=torch.int64)
+    lengths = torch.empty(state.batch, device=ids.device, dtype=torch.int64)
+    scores = torch.empty(state.batch, device=ids.device, dtype=torch.float32)
+    eos = -1 if eos_token_id is None else int(eos_token_id)
+    _lib.check(_lib.lib().b200b_beam_finalize(
+        state.batch, state.num_beams, eos, float(length_penalty), int(steps), ids.data_ptr(), ids.stride(0),
+        C.byref(state.struct), out.data_ptr(), out.stride(0), lengths.data_ptr(), scores.data_ptr(), _stream_ptr()),
+        "beam_finalize")
+    return out, lengths, scores
+
+
 def gemm_grad_pair(dy: torch.Tensor, w: torch.Tensor, x: torch.Tensor, *, wgrad_dtype: torch.dtype = torch.float32):
     """dX = dY W (bf16 [rows, n_in]) and dW = dY^T X ([n_out, n_in], fp32 or bf16) of one Linear through
     b200b_gemm_dual: ONE grouped persistent launch when both fit 256 x 128 pair tiles, two launches otherwise.
