@@ -451,31 +451,43 @@ int b200b_cross_entropy_bwd(const void* logits, int dtype, int64_t ld, const int
                             void* stream);
 
 /* ------------------------------------------------------------------------------------------- *
- * Temperature / top-p sampling, one token per row (csrc/sampling.cu). Replaces the sampling branch of a
- * decode step of FullModel.generate_caption(do_sample=True) (full_model.py:264-350: NaN / Inf guards,
- * logits / temperature, top-p filter, multinomial).
+ * Temperature / top-k / top-p sampling, one token per row (csrc/sampling.cu). Replaces the sampling branch of
+ * a decode step of FullModel.generate_caption(do_sample=True) (full_model.py:264-350: NaN / Inf guards,
+ * logits / temperature, top-p filter, multinomial), with Hugging Face's top-k filter between temperature and
+ * top-p (the order of generate(do_sample=True)).
  *
  * logits [rows, vocab], row pitch ld >= vocab elements (nothing beyond vocab is read), dtype 0 = f32,
  * 1 = bf16; arithmetic is fp32. For row b at decode step t:
  *  1. guards (as the greedy decode): a row containing a NaN becomes all zeros; otherwise a row containing
  *     +-Inf is clamped to [-100, 100];
  *  2. z_i = x_i / temperature (fp32 division), temperature finite and > 0;
- *  3. token i is kept iff the softmax(z) mass of the tokens with STRICTLY larger z is < top_p, top_p in
- *     (0, 1]: the sort-and-cumsum nucleus rule, except that tokens tied at the threshold are kept together;
- *     the maximum is always kept and top_p = 1 keeps every token;
+ *  3a. top-k (b200b_sample_tokens_top_k; top_k >= 0): skipped if top_k == 0 or top_k >= vocab. Otherwise let
+ *     z_(k) be the top_k-th largest z of the row, counting duplicates; token i passes iff z_i >= z_(k), so
+ *     tokens tied with the k-th value pass together (as Hugging Face's TopKLogitsWarper, which removes
+ *     scores < topk(...)[..., -1]). A NaN row is all zeros after 1: every token ties and passes;
+ *  3b. of the tokens that passed 3a, token i is kept iff the softmax(z) mass of the PASSING tokens with
+ *     STRICTLY larger z is < top_p times the mass of all passing tokens, top_p in (0, 1]: top-p on the
+ *     renormalised top-k set, the sort-and-cumsum nucleus rule except that tokens tied at the threshold are
+ *     kept together; the maximum is always kept and top_p = 1 keeps every passing token. With top_k = 0 this
+ *     is the top-p rule of b200b_sample_tokens;
  *  4. ids_out[b * ids_stride] = argmax over kept i of z_i + g_i, g_i = -ln(-ln u_i) (Gumbel-max: an exact
  *     draw from the renormalised nucleus), ties to the smallest index;
  *  5. u_i = ((w >> 8) + 0.5) * 2^-24, w = 32-bit word i % 4 of Philox4x32-10(counter = (i / 4, b, t mod 2^32,
  *     0x5a3b1e00), key = (seed low, seed high)); *seed is read from device memory when the kernel runs, so
  *     a captured graph or a sync-free loop draws new values by changing it. The logs are accurate logf /
  *     log1pf (u is carried exactly as u below 1/2 and as 1 - u above).
- * The mass comparisons of 3 use exp(z - zmax) in 2^-40 fixed point (relative error of a mass below 2e-5).
+ * The top-k threshold of 3a is exact (a radix select by count over the z values). The mass comparisons of 3b
+ * use exp(z - zmax) in 2^-40 fixed point (relative error of a mass below 2e-5).
  * Limits: vocab <= 8 * (180224 / e) = 360448 (f32) / 720896 (bf16) tokens -- a row is split over a cluster
  * of at most 8 CTAs holding 176 KiB of it each -- else B200B_ERR_SHAPE, as for rows < 1 or vocab < 1.
  * B200B_ERR_ARG: a null pointer, dtype not 0 / 1, ld < vocab, temperature <= 0 or not finite, top_p
- * outside (0, 1]. The cluster size is 1, 2, 4 or 8: the fewest CTAs the row fits, doubled while
+ * outside (0, 1], top_k < 0. The cluster size is 1, 2, 4 or 8: the fewest CTAs the row fits, doubled while
  * rows * CTAs is below the SM count and each CTA keeps >= 4096 tokens.
+ * b200b_sample_tokens is b200b_sample_tokens_top_k with top_k = 0 (no top-k filter).
  * ------------------------------------------------------------------------------------------- */
+int b200b_sample_tokens_top_k(const void* logits, int dtype, int64_t ld, int64_t rows, int64_t vocab,
+                              float temperature, int64_t top_k, float top_p, const unsigned long long* seed,
+                              int64_t step, int64_t* ids_out, int64_t ids_stride, void* stream);
 int b200b_sample_tokens(const void* logits, int dtype, int64_t ld, int64_t rows, int64_t vocab, float temperature,
                         float top_p, const unsigned long long* seed, int64_t step, int64_t* ids_out,
                         int64_t ids_stride, void* stream);
@@ -516,7 +528,7 @@ int b200b_sample_tokens(const void* logits, int dtype, int64_t ld, int64_t rows,
  *  N = powf(n, alpha) in fp32, clamped to [FLT_MIN, FLT_MAX] (so no score is NaN for any finite alpha).
  *  after the last step (b200b_beam_finalize, n = steps): for each image that is not done, running beams
  *  k = 0..K-1 are offered in that order with score s_k / N and length n; the result is the finished hypothesis
- *  with the best score, ties to the one added first. A hypothesis that ended in EOS at step t has caption length
+ *  with the best score, ties to the one added first (b200b_beam_finalize_top: the N best, in that order). A hypothesis that ended in EOS at step t has caption length
  *  t + 1 (BOS + t tokens; the EOS at position t + 1 is not part of it).
  *  V >= 2 is required, so the first 2K always hold at least K candidates that are not EOS.
  *
@@ -554,11 +566,19 @@ int b200b_beam_step(const void* logits, int dtype, int64_t ld, int64_t batch, in
                     int64_t eos, float length_penalty, int early_stopping, int64_t step, const int64_t* ids,
                     int64_t* ids_next, int64_t ld_ids, int64_t* parents, const b200b_beam_state* state,
                     void* workspace, size_t workspace_bytes, void* stream);
-/* The "after the last step" rule for `steps` >= 1 steps, without changing the state. ids [R][ld_ids] holds the
- * running beams (positions 0..steps). out_ids int64 [batch][ld_out]: positions 0..steps of the result, with
- * max(eos, 0) after its length; out_len int64 [batch]: its caption length + 1 (ids[b, 1:out_len[b]] is the
- * caption); out_score f32 [batch]: its normalised score. B200B_ERR_ARG: a null pointer, K outside [1, 8],
- * eos < -1, ld_ids, ld_hyp or ld_out < steps + 1, alpha not finite; B200B_ERR_SHAPE: batch < 1, steps < 1. */
+/* The "after the last step" rule for `steps` >= 1 steps, without changing the state, returning the
+ * num_return = N best hypotheses of each image (1 <= N <= K). ids [R][ld_ids] holds the running beams
+ * (positions 0..steps). After the offers of the rule, image b's finished set holds K entries (an image that is
+ * not done has just offered K beams to it; a done image already holds K), so its N best always exist; they go
+ * to rows b * N + j, j = 0..N-1, by score descending, ties to the one added first (j = 0 is the result of the
+ * rule above). out_ids int64 [batch * N][ld_out]: positions 0..steps of each, with max(eos, 0) after its length;
+ * out_len int64 [batch * N]: its caption length + 1 (ids[r, 1:out_len[r]] is the caption); out_score f32
+ * [batch * N]: its normalised score. B200B_ERR_ARG: a null pointer, K outside [1, 8], N outside [1, K],
+ * eos < -1, ld_ids, ld_hyp or ld_out < steps + 1, alpha not finite; B200B_ERR_SHAPE: batch < 1, steps < 1.
+ * b200b_beam_finalize is b200b_beam_finalize_top with N = 1. */
+int b200b_beam_finalize_top(int64_t batch, int num_beams, int num_return, int64_t eos, float length_penalty,
+                            int64_t steps, const int64_t* ids, int64_t ld_ids, const b200b_beam_state* state,
+                            int64_t* out_ids, int64_t ld_out, int64_t* out_len, float* out_score, void* stream);
 int b200b_beam_finalize(int64_t batch, int num_beams, int64_t eos, float length_penalty, int64_t steps,
                         const int64_t* ids, int64_t ld_ids, const b200b_beam_state* state, int64_t* out_ids,
                         int64_t ld_out, int64_t* out_len, float* out_score, void* stream);

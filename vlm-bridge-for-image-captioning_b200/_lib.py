@@ -155,6 +155,9 @@ def _declare(lib) -> None:
     lib.b200b_sample_tokens.restype = C.c_int
     lib.b200b_sample_tokens.argtypes = [C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_int64, C.c_float, C.c_float,
                                         C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]
+    lib.b200b_sample_tokens_top_k.restype = C.c_int
+    lib.b200b_sample_tokens_top_k.argtypes = [C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_int64, C.c_float, C.c_int64,
+                                              C.c_float, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]
     lib.b200b_beam_step_workspace_bytes.restype = C.c_size_t
     lib.b200b_beam_step_workspace_bytes.argtypes = [C.c_int64, C.c_int]
     lib.b200b_beam_step.restype = C.c_int
@@ -165,6 +168,10 @@ def _declare(lib) -> None:
     lib.b200b_beam_finalize.argtypes = [C.c_int64, C.c_int, C.c_int64, C.c_float, C.c_int64, C.c_void_p, C.c_int64,
                                         C.POINTER(BeamState), C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
                                         C.c_void_p]
+    lib.b200b_beam_finalize_top.restype = C.c_int
+    lib.b200b_beam_finalize_top.argtypes = [C.c_int64, C.c_int, C.c_int, C.c_int64, C.c_float, C.c_int64, C.c_void_p,
+                                            C.c_int64, C.POINTER(BeamState), C.c_void_p, C.c_int64, C.c_void_p,
+                                            C.c_void_p, C.c_void_p]
     lib.b200b_gemm_dual.restype = C.c_int
     lib.b200b_gemm_dual.argtypes = [C.POINTER(GemmArgs), C.POINTER(GemmArgs), C.c_void_p]
     lib.b200b_gemm_set_dual.restype = C.c_int

@@ -461,13 +461,18 @@ __global__ void __launch_bounds__(kSelThreads, 1)
   }
 }
 
+// finished entry i of an image before entry j: score desc, then added first (seq asc)
+__device__ __forceinline__ bool hyp_before(const float* hs, const int* hq, int i, int j) {
+  return hs[i] > hs[j] || (hs[i] == hs[j] && hq[i] < hq[j]);
+}
+
 __global__ void __launch_bounds__(kSelThreads, 1)
-    beam_finalize_kernel(int K, long long eos, float alpha, int steps, const long long* __restrict__ ids,
+    beam_finalize_kernel(int K, int N, long long eos, float alpha, int steps, const long long* __restrict__ ids,
                          long long ld_ids, b200b_beam_state st, long long* __restrict__ out_ids, long long ld_out,
                          long long* __restrict__ out_len, float* __restrict__ out_score) {
   __shared__ float hs[kBeamMaxK];
   __shared__ int hl[kBeamMaxK], hq[kBeamMaxK], src[kBeamMaxK];
-  __shared__ int best_src, best_len;
+  __shared__ int sel[kBeamMaxK];   // sel[r]: the slot of the r-th best hypothesis, in [0, K)
   const int b = blockIdx.x, tid = threadIdx.x;
   const long long row0 = (long long)b * K;
 
@@ -487,21 +492,32 @@ __global__ void __launch_bounds__(kSelThreads, 1)
         if (slot >= 0) src[slot] = K + k;   // running beam k
       }
     }
-    const int filled = min(count, K);   // >= 1: an image that is not done offered K beams to its set
-    int w = 0;
-    for (int j = 1; j < filled; ++j)
-      if (hs[j] > hs[w] || (hs[j] == hs[w] && hq[j] < hq[w])) w = j;
-    best_src = src[w];
-    best_len = hl[w];
-    out_len[b] = hl[w];
-    out_score[b] = hs[w];
+    // filled is K after the offers, and a done image holds K; clamped to [1, K] whatever the state holds. The N best
+    // by selection (each pick is a slot not picked before, so sel is a list of distinct slots in [0, filled) for
+    // N <= filled; a corrupt state with fewer filled slots repeats the last pick).
+    const int filled = max(min(count, K), 1);
+    unsigned used = 0;
+    for (int r = 0; r < N; ++r) {
+      int w = -1;
+      for (int j = 0; j < filled; ++j)
+        if (!(used >> j & 1u) && (w < 0 || hyp_before(hs, hq, j, w))) w = j;
+      if (w < 0) w = sel[r - 1];   // r >= 1 here: filled >= 1 slots are free at r = 0
+      used |= 1u << w;
+      sel[r] = w;
+      out_len[(long long)b * N + r] = hl[w];
+      out_score[(long long)b * N + r] = hs[w];
+    }
   }
   __syncthreads();
-  // best_src < K: slot best_src of this image's finished set; else running beam best_src - K (in [0, K))
-  const long long* srow = best_src < K ? reinterpret_cast<const long long*>(st.hyp_ids) + (row0 + best_src) * st.ld_hyp
-                                       : ids + (row0 + best_src - K) * ld_ids;
   const long long pad = eos >= 0 ? eos : 0;
-  for (int j = tid; j <= steps; j += kSelThreads) out_ids[(long long)b * ld_out + j] = j < best_len ? srow[j] : pad;
+  for (int r = 0; r < N; ++r) {
+    // s < K: slot s of this image's finished set; else running beam s - K (in [0, K))
+    const int s = src[sel[r]], len = hl[sel[r]];
+    const long long* srow = s < K ? reinterpret_cast<const long long*>(st.hyp_ids) + (row0 + s) * st.ld_hyp
+                                  : ids + (row0 + s - K) * ld_ids;
+    long long* drow = out_ids + ((long long)b * N + r) * ld_out;
+    for (int j = tid; j <= steps; j += kSelThreads) drow[j] = j < len ? srow[j] : pad;
+  }
 }
 
 template <bool BF16, int CS>
@@ -647,16 +663,20 @@ extern "C" int b200b_beam_step(const void* logits, int dtype, int64_t ld, int64_
   return check_launch("beam_select", stream);
 }
 
-extern "C" int b200b_beam_finalize(int64_t batch, int num_beams, int64_t eos, float length_penalty, int64_t steps,
-                                   const int64_t* ids, int64_t ld_ids, const b200b_beam_state* state,
-                                   int64_t* out_ids, int64_t ld_out, int64_t* out_len, float* out_score,
-                                   void* stream_) {
+extern "C" int b200b_beam_finalize_top(int64_t batch, int num_beams, int num_return, int64_t eos,
+                                       float length_penalty, int64_t steps, const int64_t* ids, int64_t ld_ids,
+                                       const b200b_beam_state* state, int64_t* out_ids, int64_t ld_out,
+                                       int64_t* out_len, float* out_score, void* stream_) {
   if (!ids || !out_ids || !out_len || !out_score || !state_ok(state)) {
     set_last_error("beam_finalize: null pointer");
     return B200B_ERR_ARG;
   }
   if (num_beams < 1 || num_beams > kBeamMaxK) {
     set_last_error("beam_finalize: num_beams must be in [1, %d]", kBeamMaxK);
+    return B200B_ERR_ARG;
+  }
+  if (num_return < 1 || num_return > num_beams) {
+    set_last_error("beam_finalize: num_return must be in [1, num_beams]");
     return B200B_ERR_ARG;
   }
   if (batch < 1 || batch > 0x7fffffffLL / kBeamMaxK || steps < 1 || steps > 0x7ffffffeLL) {
@@ -673,7 +693,7 @@ extern "C" int b200b_beam_finalize(int64_t batch, int num_beams, int64_t eos, fl
   }
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
   cudaError_t e = launch_pdl(kPdlRows, beam_finalize_kernel, dim3((unsigned)batch), dim3(kSelThreads), 0, stream,
-                             num_beams, (long long)eos, length_penalty, (int)steps,
+                             num_beams, num_return, (long long)eos, length_penalty, (int)steps,
                              reinterpret_cast<const long long*>(ids), (long long)ld_ids, *state,
                              reinterpret_cast<long long*>(out_ids), (long long)ld_out,
                              reinterpret_cast<long long*>(out_len), out_score);
@@ -682,4 +702,12 @@ extern "C" int b200b_beam_finalize(int64_t batch, int num_beams, int64_t eos, fl
     return (int)e;
   }
   return check_launch("beam_finalize", stream);
+}
+
+extern "C" int b200b_beam_finalize(int64_t batch, int num_beams, int64_t eos, float length_penalty, int64_t steps,
+                                   const int64_t* ids, int64_t ld_ids, const b200b_beam_state* state,
+                                   int64_t* out_ids, int64_t ld_out, int64_t* out_len, float* out_score,
+                                   void* stream) {
+  return b200b_beam_finalize_top(batch, num_beams, 1, eos, length_penalty, steps, ids, ld_ids, state, out_ids, ld_out,
+                                 out_len, out_score, stream);
 }

@@ -5,14 +5,19 @@
 //
 // Here one row is split over a cluster of CS CTAs (csrc/sampling.cu, sample_cluster_size): each CTA copies its
 // slice of the row from HBM into shared memory once, and every later pass runs on chip; the per-CTA partials
-// (row max and guard flags, mass histograms, the final argmax) are combined through distributed shared memory.
-// The rule (b200_bridge.h, b200b_sample_tokens):
+// (row max and guard flags, count and mass histograms, the final argmax) are combined through distributed shared memory.
+// The rule (b200_bridge.h, b200b_sample_tokens_top_k):
 //   1. guards: a row with a NaN becomes all zeros; else a row with an Inf is clamped to [-100, 100];
 //   2. z = x / T in fp32;
-//   3. token i is kept iff the softmax mass of the tokens with strictly larger z is < top_p; the threshold is a
-//      radix select BY MASS over an order-preserving 32-bit image of z: three histogram passes (11 + 11 + 10 bits)
-//      of exp(z - zmax) in 2^-40 fixed point (integer adds: the same sums in any order, so the choice is
-//      deterministic and identical in every CTA of the cluster); skipped when top_p == 1;
+//   3a. 0 < top_k < V: token i passes iff z_i >= the k-th largest z (duplicates counted, ties pass together); the
+//      threshold is a radix select BY COUNT over an order-preserving 32-bit image of z: three histogram passes
+//      (11 + 11 + 10 bits) of token counts, combined over the cluster in rank order (integers: every CTA picks the
+//      same threshold); skipped when top_k == 0 or top_k >= V;
+//   3b. of the tokens that passed 3a, token i is kept iff the softmax mass of the passing tokens with strictly
+//      larger z is < top_p times the mass of all passing tokens; the threshold is the same radix select BY MASS:
+//      three histogram passes of exp(z - zmax) in 2^-40 fixed point over the passing keys (integer adds: the same
+//      sums in any order, so the choice is deterministic and identical in every CTA of the cluster); skipped when
+//      top_p == 1;
 //   4. argmax over kept tokens of z + g, g = -ln(-ln u) (Gumbel-max: an exact draw from the renormalised nucleus),
 //      ties to the smallest index; u from Philox4x32-10 as documented in the header.
 #include <math.h>
@@ -76,7 +81,7 @@ __device__ __forceinline__ float samp_f(T v) {
 template <bool BF16, int CS>
 __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(kSampThreads, 1)
     sample_kernel(const void* __restrict__ logits, long long ld, long long vocab, long long slice, float temperature,
-                  float top_p, const unsigned long long* __restrict__ seed_ptr, uint32_t step,
+                  uint32_t top_k, float top_p, const unsigned long long* __restrict__ seed_ptr, uint32_t step,
                   long long* __restrict__ ids_out, long long ids_stride) {
   using T = typename std::conditional<BF16, __nv_bfloat16, float>::type;
   constexpr int kVec = 16 / (int)sizeof(T);
@@ -169,9 +174,14 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(kSampThreads, 1)
   };
   const float zmax = (nan_row ? 0.0f : (inf_row ? fminf(fmaxf(gmax, -100.0f), 100.0f) : gmax)) / temperature;
 
-  // ---- nucleus threshold: the smallest present key k with mass(key > k) < top_p * S ----
-  uint32_t kth = 0;   // top_p == 1: every token is kept
-  if (top_p < 1.0f) {
+  // ---- thresholds. kth: tokens with samp_key(z) >= kth are kept (0 keeps every token: keys are >= 0x007FFFFF).
+  // kth_k: the top-k threshold (0: no top-k filter). The nucleus: the smallest present key k with
+  // mass(key > k) < top_p * S, where its histograms count only keys >= kth_k (S: their mass), so every picked bin
+  // holds such a key and the nucleus threshold ends >= kth_k. TopkFilter::value adds the `key >= kth_k` test to the
+  // mass pass (a separate instantiation: the top_k == 0 path runs the loop without it).
+  uint32_t kth = 0, kth_k = 0;
+  auto nucleus = [&](auto topk_filter) {
+    using TopkFilter = decltype(topk_filter);
     uint32_t prefix = 0;
     unsigned long long above = 0;   // mass of the tokens whose key lies above the current prefix range
     double limit = 0.0;
@@ -188,7 +198,7 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(kSampThreads, 1)
       for (int i = tid; i < n; i += kSampThreads) {
         const float z = zof(xs[i]);
         const uint32_t k = samp_key(z);
-        if ((k & pmask) == prefix) {
+        if ((k & pmask) == prefix && (!TopkFilter::value || k >= kth_k)) {
           const uint32_t d = (k >> shift) & dmask;
           const unsigned long long m = __float2ull_rz(ex2_approx((z - zmax) * kSampLog2e) * kSampMassOne);
           // a 64-bit shared atomic add is a compare-and-swap loop, and logits crowd into a few exponent bins:
@@ -264,6 +274,73 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(kSampThreads, 1)
       if (level == 2) kth = prefix;
       __syncthreads();   // sel_above / red_u are rewritten by the next level
     }
+  };
+
+  // ---- top-k threshold kth_k: the key of the top_k-th largest z, counting duplicates ----
+  if (top_k != 0) {
+    uint32_t prefix = 0, above = 0;   // tokens whose key lies above the current prefix range
+    for (int level = 0; level < 3; ++level) {
+      const int shift = level == 0 ? 21 : (level == 1 ? 10 : 0);
+      const uint32_t pmask = level == 0 ? 0u : (level == 1 ? 0xFFE00000u : 0xFFFFFC00u);
+      const uint32_t dmask = level == 2 ? 0x3FFu : 0x7FFu;
+      for (int b = tid; b < kSampBins; b += kSampThreads) hcnt[b] = 0;
+      __syncthreads();
+      for (int i = tid; i < n; i += kSampThreads) {
+        const uint32_t k = samp_key(zof(xs[i]));
+        if ((k & pmask) == prefix) atomicAdd(&hcnt[(k >> shift) & dmask], 1u);
+      }
+      cluster.sync();
+      uint32_t cc[kSampBinsPerThread];
+#pragma unroll
+      for (int j = 0; j < kSampBinsPerThread; ++j) cc[j] = 0;
+      for (int r = 0; r < CS; ++r) {
+        const uint32_t* pc = cluster.map_shared_rank(hcnt, r);
+#pragma unroll
+        for (int j = 0; j < kSampBinsPerThread; ++j) cc[j] += pc[tid * kSampBinsPerThread + j];
+      }
+      cluster.sync();   // every CTA has read this CTA's histogram before the next level clears it
+      uint32_t tot = 0;
+#pragma unroll
+      for (int j = 0; j < kSampBinsPerThread; ++j) tot += cc[j];
+      uint32_t suf = tot;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const uint32_t t = __shfl_down_sync(0xffffffffu, suf, o);
+        if (lane + o < 32) suf += t;
+      }
+      if (lane == 0) red_m[warp] = suf;
+      __syncthreads();
+      uint32_t higher = suf - tot;
+      for (int w = warp + 1; w < kSampThreads / 32; ++w) higher += (uint32_t)red_m[w];
+      // the one bin with count(key above it) < top_k <= count(key above it) + its count
+      uint32_t pick = 0xFFFFFFFFu, pick_above = 0;
+      uint32_t a = above + higher;
+#pragma unroll
+      for (int j = kSampBinsPerThread - 1; j >= 0; --j) {
+        if (a < top_k && a + cc[j] >= top_k) {
+          pick = (uint32_t)(tid * kSampBinsPerThread + j);
+          pick_above = a;
+        }
+        a += cc[j];
+      }
+      const uint32_t wpick = __reduce_min_sync(0xffffffffu, pick);
+      if (lane == 0) red_u[warp] = wpick;
+      __syncthreads();
+      uint32_t bpick = 0xFFFFFFFFu;
+      for (int w = 0; w < kSampThreads / 32; ++w) bpick = min(bpick, red_u[w]);
+      if (pick == bpick && pick != 0xFFFFFFFFu) sel_above = pick_above;
+      __syncthreads();
+      // a bin always qualifies (top_k < V tokens in all); guard regardless
+      if (bpick == 0xFFFFFFFFu) break;
+      prefix |= bpick << shift;
+      above = (uint32_t)sel_above;
+      if (level == 2) kth_k = prefix;
+      __syncthreads();   // sel_above / red_u / red_m are rewritten by the next level
+    }
+    kth = kth_k;
+    if (top_p < 1.0f) nucleus(std::true_type{});
+  } else if (top_p < 1.0f) {
+    nucleus(std::false_type{});
   }
 
   // ---- draw: argmax over the kept tokens of z + Gumbel noise ----
@@ -349,8 +426,8 @@ int sample_cluster_size(long long rows, long long vocab, int esz, int sms, long 
 
 template <bool BF16, int CS>
 static int sample_launch(const void* logits, long long ld, long long rows, long long vocab, long long slice,
-                         float temperature, float top_p, const unsigned long long* seed, uint32_t step,
-                         long long* ids_out, long long ids_stride, cudaStream_t stream) {
+                         float temperature, uint32_t top_k, float top_p, const unsigned long long* seed,
+                         uint32_t step, long long* ids_out, long long ids_stride, cudaStream_t stream) {
   auto kern = sample_kernel<BF16, CS>;
   const size_t smem = (size_t)slice * (BF16 ? 2 : 4);
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -359,7 +436,7 @@ static int sample_launch(const void* logits, long long ld, long long rows, long 
     return (int)e;
   }
   e = launch_pdl(kPdlRows, kern, dim3((unsigned)(rows * CS)), dim3(kSampThreads), smem, stream, logits, ld, vocab,
-                 slice, temperature, top_p, seed, step, ids_out, ids_stride);
+                 slice, temperature, top_k, top_p, seed, step, ids_out, ids_stride);
   if (e != cudaSuccess) {
     set_last_error("sample_tokens: launch failed: %s", cudaGetErrorString(e));
     return (int)e;
@@ -371,9 +448,10 @@ static int sample_launch(const void* logits, long long ld, long long rows, long 
 
 using namespace b200b;
 
-extern "C" int b200b_sample_tokens(const void* logits, int dtype, int64_t ld, int64_t rows, int64_t vocab,
-                                   float temperature, float top_p, const unsigned long long* seed, int64_t step,
-                                   int64_t* ids_out, int64_t ids_stride, void* stream_) {
+extern "C" int b200b_sample_tokens_top_k(const void* logits, int dtype, int64_t ld, int64_t rows, int64_t vocab,
+                                         float temperature, int64_t top_k, float top_p,
+                                         const unsigned long long* seed, int64_t step, int64_t* ids_out,
+                                         int64_t ids_stride, void* stream_) {
   if (!logits || !seed || !ids_out) {
     set_last_error("sample_tokens: null pointer");
     return B200B_ERR_ARG;
@@ -398,6 +476,10 @@ extern "C" int b200b_sample_tokens(const void* logits, int dtype, int64_t ld, in
     set_last_error("sample_tokens: top_p must be in (0, 1]");
     return B200B_ERR_ARG;
   }
+  if (top_k < 0) {
+    set_last_error("sample_tokens: top_k must be >= 0");
+    return B200B_ERR_ARG;
+  }
   if (rows > 0x7fffffffLL / kSampMaxCluster) {
     set_last_error("sample_tokens: too many rows");
     return B200B_ERR_SHAPE;
@@ -416,9 +498,10 @@ extern "C" int b200b_sample_tokens(const void* logits, int dtype, int64_t ld, in
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
   long long* out = reinterpret_cast<long long*>(ids_out);
   const uint32_t t = (uint32_t)step;
-#define SAMPLE_CASE(BF, C)                                                                                      \
-  if (cs == C)                                                                                                  \
-    return sample_launch<BF, C>(logits, ld, rows, vocab, slice, temperature, top_p, seed, t, out, ids_stride, \
+  const uint32_t k = top_k < vocab ? (uint32_t)top_k : 0u;   // top_k >= vocab keeps every token, as top_k == 0
+#define SAMPLE_CASE(BF, C)                                                                                         \
+  if (cs == C)                                                                                                     \
+    return sample_launch<BF, C>(logits, ld, rows, vocab, slice, temperature, k, top_p, seed, t, out, ids_stride, \
                                 stream);
   if (dtype == 1) {
     SAMPLE_CASE(true, 1) SAMPLE_CASE(true, 2) SAMPLE_CASE(true, 4) SAMPLE_CASE(true, 8)
@@ -428,4 +511,11 @@ extern "C" int b200b_sample_tokens(const void* logits, int dtype, int64_t ld, in
 #undef SAMPLE_CASE
   set_last_error("sample_tokens: no kernel for cluster size %d", cs);
   return B200B_ERR_SHAPE;
+}
+
+extern "C" int b200b_sample_tokens(const void* logits, int dtype, int64_t ld, int64_t rows, int64_t vocab,
+                                   float temperature, float top_p, const unsigned long long* seed, int64_t step,
+                                   int64_t* ids_out, int64_t ids_stride, void* stream) {
+  return b200b_sample_tokens_top_k(logits, dtype, ld, rows, vocab, temperature, 0, top_p, seed, step, ids_out,
+                                   ids_stride, stream);
 }

@@ -5,9 +5,9 @@ start from BOS, every step embeds the whole prefix, runs the bridge over it (the
 self-attention is non-causal, so earlier positions change when a token is appended and the prefix
 must be recomputed -- only the image's K/V are exactly cacheable), feeds the result to the language
 model, takes `argmax` of the last position's logits (NaN logits -> zeros, Inf logits -> clamped to
-+-100, as :270-283) and appends it. With `do_sample=True` the token is drawn instead (temperature, top-p
-nucleus, one fused kernel per step: `ops.sample_tokens`, csrc/sampling.cu), as the sampling branch
-(:264-350) does.
++-100, as :270-283) and appends it. With `do_sample=True` the token is drawn instead (temperature, top-k,
+top-p nucleus, one fused kernel per step: `ops.sample_tokens`, csrc/sampling.cu), as the sampling branch
+(:264-350) does; `num_return_sequences` draws several captions per image over one shared cache of the image.
 
 The reference loop is batch-1 and synchronises with the host up to three times per step
 (`next_token.item()`, :317,355-366). Here B images decode together with no host synchronisation:
@@ -22,6 +22,7 @@ independent reference runs produce (generation is deterministic and rows never i
 from __future__ import annotations
 
 import math
+import numbers
 from typing import Callable, Optional
 
 import torch
@@ -111,8 +112,8 @@ def greedy_decode(bridge, vision_features: torch.Tensor, embed_fn: Callable[[tor
                   kv_cache: Optional[VisionKVCache] = None, use_cache: bool = True,
                   step_graphs: Optional[DecodeStepGraphs] = None, use_graphs: bool = False,
                   cache_positions: bool = True, precision: str = "bf16", refill_cache: bool = False,
-                  do_sample: bool = False, temperature: float = 1.0, top_p: float = 1.0,
-                  generator: Optional[torch.Generator] = None):
+                  do_sample: bool = False, temperature: float = 1.0, top_p: float = 1.0, top_k: int = 0,
+                  num_return_sequences: int = 1, generator: Optional[torch.Generator] = None):
     """Returns (ids [B, 1 + max_new_tokens] int64 incl. BOS, lengths [B] int64): row b's caption is
     ids[b, 1:lengths[b]] (EOS excluded); positions from lengths[b] on are what the lock-step loop kept
     generating and are to be ignored. `use_graphs` replays one captured CUDA graph of the bridge per
@@ -134,19 +135,40 @@ def greedy_decode(bridge, vision_features: torch.Tensor, embed_fn: Callable[[tor
     stated in include/b200_bridge.h). One 64-bit seed per call is drawn on the device from `generator` (a CUDA
     generator on the images' device; None = that device's default generator), so the loop never waits for the
     host and the same generator state gives the same captions. The step graphs still capture only the bridge;
-    the sampler runs after each replay. Bad `temperature` / `top_p` values or a generator on another device
-    raise ValueError before any kernel runs."""
+    the sampler runs after each replay. `top_k` > 0 keeps, before the nucleus, only the tokens whose z is at least
+    the top_k-th largest (ties kept together; 0 = off), as generate(do_sample=True, top_k=...) applies it between
+    temperature and top-p.
+
+    `num_return_sequences` = N > 1 (do_sample=True only, N <= 8) draws N captions per image over ONE cache of the
+    images (`VisionKVCache(..., beams=N)`: each image's K/V is read once per step for all its N rows).
+    `embed_fn` / `lm_fn` then see B*N rows in [B][N] order, and the results have B*N rows: row b*N + j is sample j
+    of image b (the order of Hugging Face's repeat_interleave), drawn with the noise of row b*N + j of a sampled
+    decode over `vision_features.repeat_interleave(N, 0)`. A `kv_cache` passed in must be built with beams=N.
+
+    Bad `temperature` / `top_p` / `top_k` values, a `num_return_sequences` outside [1, 8] or above 1 without
+    do_sample=True or use_cache=True, or a generator on another device raise ValueError before any kernel runs."""
     was_training = bridge.training
     bridge.eval()
     try:
         B = vision_features.shape[0]
         dev = vision_features.device
+        if isinstance(num_return_sequences, bool) or not isinstance(num_return_sequences, numbers.Integral):
+            raise ValueError(f"num_return_sequences must be an int, got {num_return_sequences!r}")
+        N = int(num_return_sequences)
+        if not 1 <= N <= 8:
+            raise ValueError(f"num_return_sequences must be in [1, 8], got {N}")
+        if N > 1 and not do_sample:
+            raise ValueError("num_return_sequences > 1 needs do_sample=True (use beam_search_decode for the N best beams)")
+        if N > 1 and not use_cache:
+            raise ValueError("num_return_sequences > 1 shares one VisionKVCache per image: use_cache must stay True")
         if do_sample:
             temperature, top_p = float(temperature), float(top_p)
             if not (math.isfinite(temperature) and temperature > 0.0):
                 raise ValueError(f"temperature must be finite and > 0, got {temperature}")
             if not (0.0 < top_p <= 1.0):
                 raise ValueError(f"top_p must be in (0, 1], got {top_p}")
+            if isinstance(top_k, bool) or not isinstance(top_k, numbers.Integral) or top_k < 0:
+                raise ValueError(f"top_k must be an int >= 0, got {top_k!r}")
             if dev.type != "cuda":
                 raise ValueError("do_sample=True needs the images on a CUDA device")
             gdev = None if generator is None else torch.device(generator.device)
@@ -155,7 +177,8 @@ def greedy_decode(bridge, vision_features: torch.Tensor, embed_fn: Callable[[tor
             if gdev is not None and gdev != dev:
                 raise ValueError(f"generator is on {generator.device}, the images on {dev}")
         kv_cache, step_graphs = _decode_setup(bridge, vision_features, max_new_tokens, kv_cache, use_cache, step_graphs,
-                                              use_graphs, precision, refill_cache)
+                                              use_graphs, precision, refill_cache, beams=N)
+        B *= N   # rows: N per image, [B][N]
         ids = torch.empty((B, 1 + max_new_tokens), dtype=torch.long, device=dev)
         ids[:, 0] = bos_token_id
         if do_sample:
@@ -174,7 +197,7 @@ def greedy_decode(bridge, vision_features: torch.Tensor, embed_fn: Callable[[tor
             if do_sample:
                 if logits.dtype not in (torch.float32, torch.bfloat16) or logits.stride(-1) != 1:
                     logits = logits.float().contiguous()
-                ops.sample_tokens(logits, temperature=temperature, top_p=top_p, seed=seed, step=step,
+                ops.sample_tokens(logits, temperature=temperature, top_p=top_p, top_k=int(top_k), seed=seed, step=step,
                                   out=ids[:, step + 1])
                 continue
             logits = logits.float()
@@ -201,7 +224,7 @@ def beam_search_decode(bridge, vision_features: torch.Tensor, embed_fn: Callable
                        eos_token_id: Optional[int] = None, max_new_tokens: int = 50, length_penalty: float = 1.0,
                        early_stopping: bool = False, kv_cache: Optional[VisionKVCache] = None,
                        step_graphs: Optional[DecodeStepGraphs] = None, use_graphs: bool = False,
-                       precision: str = "bf16", refill_cache: bool = False):
+                       precision: str = "bf16", refill_cache: bool = False, num_return_sequences: int = 1):
     """Beam search over B images with `num_beams` = K beams each (generate(num_beams=K) of the Hugging Face stack the
     language model comes from; the rule, including where it differs from Hugging Face, is stated in
     include/b200_bridge.h at b200b_beam_step). Returns (ids [B, 1 + max_new_tokens] int64 incl. BOS, lengths [B]
@@ -215,11 +238,18 @@ def beam_search_decode(bridge, vision_features: torch.Tensor, embed_fn: Callable
     reorders the cached position rows by the chosen parents; nothing waits for the host, eagerly or with step
     graphs (`use_graphs` / `step_graphs`, as in `greedy_decode`). All beams run `max_new_tokens` steps in lock-step:
     an image whose search is done keeps its result while its rows keep flowing through the bridge.
-    `num_beams` outside [1, 8], a non-finite `length_penalty`, a `kv_cache` built for another number of beams or a
-    `precision` other than "bf16" / "fp32" raise ValueError before any kernel runs."""
+    `num_return_sequences` = N returns each image's N best hypotheses (generate(num_beams=K, num_return_sequences=N)):
+    the outputs then have B*N rows, row b*N + j the j-th best of image b (scores non-increasing in j; j = 0 is the
+    N = 1 result).
+    `num_beams` outside [1, 8], `num_return_sequences` outside [1, num_beams], a non-finite `length_penalty`, a
+    `kv_cache` built for another number of beams or a `precision` other than "bf16" / "fp32" raise ValueError before
+    any kernel runs."""
     K = int(num_beams)
     if not 1 <= K <= 8:
         raise ValueError(f"num_beams must be in [1, 8], got {num_beams}")
+    if isinstance(num_return_sequences, bool) or not isinstance(num_return_sequences, numbers.Integral) or \
+            not 1 <= num_return_sequences <= K:
+        raise ValueError(f"num_return_sequences must be an int in [1, num_beams = {K}], got {num_return_sequences!r}")
     length_penalty = float(length_penalty)
     if not math.isfinite(length_penalty):
         raise ValueError(f"length_penalty must be finite, got {length_penalty}")
@@ -253,6 +283,7 @@ def beam_search_decode(bridge, vision_features: torch.Tensor, embed_fn: Callable
                           length_penalty=length_penalty, early_stopping=early_stopping)
             kv_cache.reorder_beams(parents)
             ids, ids_next = ids_next, ids
-        return ops.beam_finalize(ids, state, steps=T, eos_token_id=eos_token_id, length_penalty=length_penalty)
+        return ops.beam_finalize(ids, state, steps=T, eos_token_id=eos_token_id, length_penalty=length_penalty,
+                                 num_return_sequences=int(num_return_sequences))
     finally:
         bridge.train(was_training)

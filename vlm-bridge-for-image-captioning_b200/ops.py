@@ -280,10 +280,12 @@ def attention_decode_tc(q: torch.Tensor, kv_tc: torch.Tensor, *, block_index: in
 
 
 def sample_tokens(logits: torch.Tensor, *, temperature: float, top_p: float, seed: torch.Tensor, step: int,
-                  out: torch.Tensor | None = None) -> torch.Tensor:
+                  out: torch.Tensor | None = None, top_k: int = 0) -> torch.Tensor:
     """One token per row of logits [rows, V] (fp32 or bf16, unit inner stride, any row pitch): NaN / Inf guards,
-    z = logits / temperature, the top-p nucleus (tokens whose strictly-larger-z mass is < top_p), then the
-    Gumbel-max draw keyed by Philox4x32-10 of (seed, row, step); the rule is stated in b200_bridge.h.
+    z = logits / temperature, the top-k filter (top_k > 0: tokens with z >= the top_k-th largest z; 0 or >= V: off),
+    the top-p nucleus of what passed (tokens whose strictly-larger-z mass is < top_p times the passing mass), then
+    the Gumbel-max draw keyed by Philox4x32-10 of (seed, row, step); the rule is stated in b200_bridge.h
+    (b200b_sample_tokens_top_k).
     `seed` is a one-element int64 CUDA tensor read when the kernel runs. Returns `out` (int64 [rows], any
     stride; allocated when None)."""
     _need_cuda(logits, seed, out)
@@ -299,9 +301,10 @@ def sample_tokens(logits: torch.Tensor, *, temperature: float, top_p: float, see
     if out.dtype != torch.int64 or out.dim() != 1 or out.shape[0] != rows:
         raise RuntimeError("sample_tokens: `out` must be int64 [rows]")
     ld = logits.stride(0) if rows > 1 else max(logits.stride(0), vocab)
-    _lib.check(_lib.lib().b200b_sample_tokens(logits.data_ptr(), 1 if logits.dtype == torch.bfloat16 else 0, ld, rows,
-                                              vocab, float(temperature), float(top_p), seed.data_ptr(), int(step),
-                                              out.data_ptr(), out.stride(0), _stream_ptr()), "sample_tokens")
+    _lib.check(_lib.lib().b200b_sample_tokens_top_k(logits.data_ptr(), 1 if logits.dtype == torch.bfloat16 else 0, ld,
+                                                    rows, vocab, float(temperature), int(top_k), float(top_p),
+                                                    seed.data_ptr(), int(step), out.data_ptr(), out.stride(0),
+                                                    _stream_ptr()), "sample_tokens")
     return out
 
 
@@ -382,23 +385,27 @@ def beam_step(logits: torch.Tensor, ids: torch.Tensor, ids_next: torch.Tensor, p
 
 
 def beam_finalize(ids: torch.Tensor, state: BeamState, *, steps: int, eos_token_id: int | None,
-                  length_penalty: float = 1.0):
-    """The "after the last step" rule of b200b_beam_finalize over the running beams ids [batch * K, >= steps + 1]
-    after `steps` steps; the state is not changed. Returns (ids int64 [batch, 1 + steps], lengths int64 [batch],
-    scores fp32 [batch]): ids[b, 1:lengths[b]] is image b's caption, EOS excluded."""
+                  length_penalty: float = 1.0, num_return_sequences: int = 1):
+    """The "after the last step" rule of b200b_beam_finalize_top over the running beams ids [batch * K, >= steps + 1]
+    after `steps` steps; the state is not changed. Returns the N = `num_return_sequences` (in [1, K]) best hypotheses
+    of each image, best first: (ids int64 [batch * N, 1 + steps], lengths int64 [batch * N], scores fp32 [batch * N]);
+    row b * N + j is image b's j-th best, ids[r, 1:lengths[r]] its caption, EOS excluded."""
     _need_cuda(ids)
+    N = int(num_return_sequences)
+    if not 1 <= N <= state.num_beams:
+        raise ValueError(f"num_return_sequences must be in [1, num_beams = {state.num_beams}], got {num_return_sequences}")
     R = state.batch * state.num_beams
     if ids.dtype != torch.int64 or ids.dim() != 2 or ids.shape[0] != R or ids.stride(1) != 1:
         raise RuntimeError("beam_finalize: ids must be int64 [batch * K, L] with unit inner stride")
     if ids.shape[1] < int(steps) + 1:
         raise RuntimeError(f"beam_finalize: ids need >= steps + 1 = {int(steps) + 1} columns")
     _same_device("beam_finalize", ids, state.beam_scores)
-    out = torch.empty((state.batch, 1 + int(steps)), device=ids.device, dtype=torch.int64)
-    lengths = torch.empty(state.batch, device=ids.device, dtype=torch.int64)
-    scores = torch.empty(state.batch, device=ids.device, dtype=torch.float32)
+    out = torch.empty((state.batch * N, 1 + int(steps)), device=ids.device, dtype=torch.int64)
+    lengths = torch.empty(state.batch * N, device=ids.device, dtype=torch.int64)
+    scores = torch.empty(state.batch * N, device=ids.device, dtype=torch.float32)
     eos = -1 if eos_token_id is None else int(eos_token_id)
-    _lib.check(_lib.lib().b200b_beam_finalize(
-        state.batch, state.num_beams, eos, float(length_penalty), int(steps), ids.data_ptr(), ids.stride(0),
+    _lib.check(_lib.lib().b200b_beam_finalize_top(
+        state.batch, state.num_beams, N, eos, float(length_penalty), int(steps), ids.data_ptr(), ids.stride(0),
         C.byref(state.struct), out.data_ptr(), out.stride(0), lengths.data_ptr(), scores.data_ptr(), _stream_ptr()),
         "beam_finalize")
     return out, lengths, scores
